@@ -30,6 +30,12 @@ They print the same JSON line shape with their own `config.workload` (tools/benc
 
 `--impl reference` times the reference's own CPU algorithm (oracle restatement, faithful mode: per-query varint
 decode + doc-length vector + WAND, the reference's default execution) on the host cores; rank 0 only.
+
+`--dump-outputs DIR` (c2, c3) writes the top-k the last timed step handed its caller to DIR as .npy files, so that two
+builds run with the same arguments (hence the same seeded corpus and queries) can be compared output for output:
+hits_doc_id, hits_segment_ord (float64, exact) and hits_score (float32, bit for bit) of shape [queries, k], with the
+slots past a query's count set to 0; counts (float64, [queries]); query_index (float64): the batch rows written, all
+of them unless the dump would pass 64 MB, then a fixed seeded sample.
 """
 from __future__ import annotations
 
@@ -74,7 +80,12 @@ def parse_args():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-exhaustive", action="store_true", help="skip the exhaustive (bm25) leg and its roofline")
     ap.add_argument("--no-pruned", action="store_true", help=argparse.SUPPRESS)  # (round-1 flag: same as --no-exhaustive)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step to DIR/<name>.npy (c2, c3)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.config not in ("c2", "c3")):
+        ap.error("--dump-outputs covers --impl ours with --config c2 or c3")
     cfg = {"c2": (10_000_000, 4096, 10), "c3": (8_841_823, 1024, 1000), "c4": (10_000_000, 4096, 10), "c5": (0, 1024, 10)}[args.config]
     args.docs = args.docs or cfg[0]
     args.queries = args.queries or cfg[1]
@@ -165,6 +176,27 @@ class ClockSampler:
         if not sm:
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["no samples"]}
         return {"sm_mhz": float(np.median(sm)), "sm_max_mhz": float(max(mx)), "reasons": sorted(reasons), "samples": len(sm)}
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, hits: np.ndarray, counts: np.ndarray) -> None:
+    """hits [Q, k] (HIT_DTYPE) and counts [Q] as the .npy files the module docstring lists"""
+    n_q, k = hits.shape
+    bytes_per_query = k * (8 + 8 + 4) + 8 + 8
+    rows = np.arange(n_q)
+    if n_q * bytes_per_query > DUMP_LIMIT_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(n_q, DUMP_LIMIT_BYTES // bytes_per_query, replace=False))
+    hits, counts = hits[rows], counts[rows]
+    valid = np.arange(k)[None, :] < counts[:, None]
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"hits_doc_id": np.where(valid, hits["doc_id"], 0).astype(np.float64),
+              "hits_segment_ord": np.where(valid, hits["segment_ord"], 0).astype(np.float64),
+              "hits_score": np.where(valid, hits["score"], np.float32(0)).astype(np.float32),
+              "counts": counts.astype(np.float64), "query_index": rows.astype(np.float64)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 # ---- workloads ---------------------------------------------------------------------------------------------------
@@ -301,7 +333,8 @@ def main():
         return float(t.item())
 
     def time_resident(execution: str):
-        """(ms per step, kernel ms, launches per step, results, counters) of one execution with the batch resident"""
+        """(ms per step, kernel ms, launches per step, results, counters, results of the last timed step) of one execution
+        with the batch resident"""
         p = gi.prepare(qb, k, execution)
 
         def step():
@@ -317,9 +350,11 @@ def main():
         with torch.cuda.stream(stream):
             ev0.record(stream)
             for _ in range(args.steps):
-                step()
+                last = step()
             ev1.record(stream)
         barrier()
+        if world == 1:
+            last = p.fetch()  # the one-GPU step leaves its result on the device, where a caller fetches it
         c1 = gi.counters()
         ms = max_over_ranks(ev0.elapsed_time(ev1)) / args.steps
         launches = (c1["kernel_launches"] - c0["kernel_launches"]) / args.steps
@@ -339,7 +374,7 @@ def main():
             p.fetch()  # (this rank's own work counters)
         ctr = gi.counters()
         p.free()
-        return ms, kernel_ms, launches, res, ctr
+        return ms, kernel_ms, launches, res, ctr, last
 
     def time_e2e(execution: str):
         def step():
@@ -368,15 +403,17 @@ def main():
 
     # ---- headline execution ----
     sampler = ClockSampler(local_rank) if rank == 0 else None
-    ms_step, kernel_ms, launches, (got_h, got_c), ctr = time_resident(args.execution)
+    ms_step, kernel_ms, launches, (got_h, got_c), ctr, last = time_resident(args.execution)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last)
     e2e = None if args.no_e2e else time_e2e(args.execution)
 
     # ---- exhaustive leg: roofline of the scoring kernels, and the result the pruned run must reproduce byte for byte ----
     exhaustive = None
     ex_h = ex_c = None
     if args.execution != "bm25" and not args.no_exhaustive:
-        x_ms, x_kernel_ms, x_launches, (ex_h, ex_c), x_ctr = time_resident("bm25")
+        x_ms, x_kernel_ms, x_launches, (ex_h, ex_c), x_ctr, _ = time_resident("bm25")
         exhaustive = {"execution": "bm25", "value": args.queries / (x_ms / 1e3), "unit": "queries/s", "ms_per_step": x_ms,
                       "kernel_ms": x_kernel_ms, "gpu_launches": x_launches,
                       "postings_scanned": int(x_ctr["last_postings_scattered"]), "postings_verified": int(x_ctr["last_postings_verified"])}

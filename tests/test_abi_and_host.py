@@ -59,7 +59,9 @@ def test_rust_sys_crate_is_in_sync_with_the_header():
 
 
 def test_library_is_built_for_sm_100a_only():
-    out = os.popen(f"cuobjdump --list-elf {slg_build.LIB_PATH} 2>/dev/null").read()
+    import subprocess
+    cuobjdump = os.path.join(os.path.dirname(slg_build._nvcc()), "cuobjdump")  # the toolkit that built the library, on PATH or not
+    out = subprocess.run([cuobjdump, "--list-elf", slg_build.LIB_PATH], capture_output=True, text=True, check=True).stdout
     archs = set(re.findall(r"sm_\d+a?", out))
     assert archs == {"sm_100a"}, archs
 
