@@ -213,9 +213,11 @@ int32_t slg_configure(slg_index_t *, uint32_t tile_docs, uint32_t ctas_per_sm, u
  *                           (default 24; 0 = no columns)
  *   "dense_min_df"     n    ... and df >= n (default 256)
  *   "max_column_bytes" n    byte budget of the columns of one segment, largest df first (default 24 GiB)
- *   "bitmap_den"       n    terms with df * n >= doc_count and no column get a presence bitmap, one bit
- *                           per doc, for the verification's "does this list hold the doc" (default 512; 0 = none)
- *   "max_bitmap_bytes" n    byte budget of those bitmaps (default 16 GiB)
+ *   "bitmap_den"       n    terms with df * n >= doc_count (and df >= 64) and no column get a presence bitmap
+ *                           with interleaved rank, 32 bytes per 224 docs: the verification learns whether the
+ *                           list holds the doc and, if so, its position in the list from one 32-byte sector,
+ *                           without searching the list (default 512; 0 = none: every look-up searches)
+ *   "max_bitmap_bytes" n    byte budget of those bitmaps, largest df first, at most 32768 rows (default 16 GiB)
  *   "keep_positions"   1/0  keep term positions resident when a posting image carries them (default 1)
  *   "scan_kernels"     1/0  plain OR batches on the flat posting scan (default 1); 0 = the sub-tile kernels
  *   "stream_kernels"   1/0  with scan_kernels 0: exhaustive batches on the sparse pass + column pass (default 1)

@@ -212,10 +212,10 @@ int32_t finish_segment(slg_index *ix, std::unique_ptr<Segment> seg, const int64_
     SLG_CUDA(ix, cudaGetLastError());
     d.term_ub = s->term_ub.as<float>();
   }
-  // presence bitmaps for the mid-dense terms without a column: the posting scan's verification asks "does this list hold
-  // the doc" far more often than the answer is yes, and a bit test is one 32-byte sector where a search is several
+  // presence bitmaps with interleaved rank for the mid-dense terms without a column: the posting scan's verification asks
+  // "does this list hold the doc, and where", and one 32-byte sector answers both where a search reads several
   if (ix->resident_scores && ix->bitmap_den && s->doc_count && s->n_blocks) {
-    const uint32_t stride = (uint32_t)align_up(((uint64_t)s->doc_count + 31) / 32, 32);
+    const uint32_t stride = presence_row_words(s->doc_count);
     std::vector<uint32_t> cand;
     for (uint64_t t = 0; t < s->n_terms; t++) {
       const uint64_t df = s->h_df[t];
@@ -237,7 +237,19 @@ int32_t finish_segment(slg_index *ix, std::unique_ptr<Segment> seg, const int64_
       slg_fill_presence_kernel<<<dim3(64, (unsigned)cand.size()), 256, 0, st>>>(d, d_terms.as<uint32_t>(), (uint32_t)cand.size(), s->pres_bits.as<uint32_t>(), stride);
       count_launch(ix);
       SLG_CUDA(ix, cudaGetLastError());
+      DevBuf d_totals;
+      SLG_CUDA(ix, d_totals.alloc(cand.size() * 4));
+      slg_presence_rank_kernel<<<(unsigned)cand.size(), kRankThreads, 0, st>>>(s->pres_bits.as<uint32_t>(), stride, (uint32_t)cand.size(), d_totals.as<uint32_t>());
+      count_launch(ix);
+      SLG_CUDA(ix, cudaGetLastError());
+      std::vector<uint32_t> totals(cand.size());
+      SLG_CUDA(ix, cudaMemcpyAsync(totals.data(), d_totals.p, cand.size() * 4, cudaMemcpyDeviceToHost, st));
       SLG_CUDA(ix, cudaStreamSynchronize(st));
+      // every row must count exactly its list: a look-up's rank is a posting index, so a wrong count would read another posting
+      for (size_t r = 0; r < cand.size(); r++)
+        if (totals[r] != s->h_df[cand[r]])
+          return fail(ix, SLG_ERR_INVALID, "segment %u: presence bitmap of term %u counts %u docs, its list holds %u", s->ord, cand[r], totals[r],
+                      s->h_df[cand[r]]);
       s->n_bitmaps = (uint32_t)cand.size();
       d.term_bits = s->term_bits.as<int32_t>();
       d.pres_bits = s->pres_bits.as<uint32_t>();

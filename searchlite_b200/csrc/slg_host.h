@@ -182,7 +182,7 @@ struct slg_index {
   bool resident_scores = true;   // build seg.post_score at load
   uint32_t dense_den = 24;       // a term gets a dense column when df * dense_den >= doc_count; 0 = no columns (C2: 8 -> 24 took the pruned batch from 9.5 to 7.6 ms for +8.7 GB)
   uint32_t dense_min_df = 256;   // ... and df >= this
-  uint32_t bitmap_den = 512;     // a term without a column gets a presence bitmap (1 bit per doc) when df * bitmap_den >= doc_count; 0 = none
+  uint32_t bitmap_den = 512;     // a term without a column gets a presence bitmap with rank (slg_residency.cuh) when df * bitmap_den >= doc_count; 0 = none
   uint64_t max_bitmap_bytes = 16ull << 30;
   uint64_t max_column_bytes = 24ull << 30;
   uint32_t stage_cap = 1024;     // sparse pass: postings a warp stages in shared memory per span (slg_stream_kernel.cuh)

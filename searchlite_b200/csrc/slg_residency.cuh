@@ -96,7 +96,39 @@ static __global__ void slg_fill_columns_kernel(SegmentDev seg, const uint32_t *c
     col[seg.post_doc[base + i]] = seg.post_score[base + i];
 }
 
-// grid (chunks, n_rows): row r holds one bit per doc for term bm_terms[r] (rows are zero on entry)
+// ---- presence bitmaps with interleaved rank ----------------------------------------------------------------------
+// A row is an array of 32-byte units, one DRAM sector each.  Word 0 of unit u holds the number of docs the list holds
+// before doc 224u (the set bits of every earlier unit of the row); words 1..7 hold one bit per doc of [224u, 224u + 224).
+// Lists are strictly ascending, so the position of a held doc in its list is its rank: the bit and the posting index
+// come out of the same sector, and a look-up never searches post_doc.  (A 64-byte unit would halve the rank words'
+// share, 1/16 instead of 1/8, but touch two sectors per look-up.)
+constexpr uint32_t kPresUnitDocs = 224;  // docs per unit
+constexpr uint32_t kPresUnitWords = 8;
+
+__host__ __device__ inline uint32_t presence_row_words(uint32_t doc_count) {
+  return (doc_count + kPresUnitDocs - 1) / kPresUnitDocs * kPresUnitWords;
+}
+
+// does the row at word offset row_off of seg.pres_bits hold doc; if so, at = the doc's position in the term's list.  The
+// one place that reads seg.pres_bits: every kernel asks here
+__device__ __forceinline__ bool presence_lookup(const SegmentDev &seg, uint64_t row_off, uint32_t doc, uint32_t &at) {
+  const uint32_t u = doc / kPresUnitDocs, r = doc - u * kPresUnitDocs;
+  const uint4 *p = reinterpret_cast<const uint4 *>(seg.pres_bits + row_off + (uint64_t)u * kPresUnitWords);
+  const uint4 a = __ldg(p), b = __ldg(p + 1);  // (both halves of the unit's one sector)
+  const uint32_t w[kPresUnitWords] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
+  const uint32_t wi = 1u + (r >> 5), bit = r & 31u;
+  uint32_t word = 0u, n = w[0];
+#pragma unroll
+  for (uint32_t i = 1; i < kPresUnitWords; i++) {
+    if (i < wi) n += __popc(w[i]);
+    if (i == wi) word = w[i];
+  }
+  at = n + __popc(word & ((1u << bit) - 1u));
+  return (word >> bit) & 1u;
+}
+
+// grid (chunks, n_rows): the bits of row r for term bm_terms[r] (rows are zero on entry; slg_presence_rank_kernel then
+// writes the rank words)
 static __global__ void slg_fill_presence_kernel(SegmentDev seg, const uint32_t *bm_terms, uint32_t n_rows, uint32_t *bits, uint32_t stride) {
   const uint32_t r = blockIdx.y;
   if (r >= n_rows) return;
@@ -106,8 +138,54 @@ static __global__ void slg_fill_presence_kernel(SegmentDev seg, const uint32_t *
   uint32_t *row = bits + (uint64_t)r * stride;
   for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < df; i += gridDim.x * blockDim.x) {
     const uint32_t doc = d[i];
-    atomicOr(row + (doc >> 5), 1u << (doc & 31));
+    const uint32_t u = doc / kPresUnitDocs, rem = doc - u * kPresUnitDocs;
+    atomicOr(row + (uint64_t)u * kPresUnitWords + 1u + (rem >> 5), 1u << (rem & 31));
   }
+}
+
+// one CTA per row: word 0 of every unit = exclusive scan of the units' popcounts; totals[r] = the row's set bits (the
+// loader checks it against the list's df)
+constexpr uint32_t kRankThreads = 1024;
+static __global__ void __launch_bounds__(kRankThreads) slg_presence_rank_kernel(uint32_t *bits, uint32_t stride, uint32_t n_rows, uint32_t *totals) {
+  __shared__ uint32_t s_warp[kRankThreads / 32 + 1];  // exclusive prefix of every warp's units, then the tile's total
+  const uint32_t r = blockIdx.x;
+  if (r >= n_rows) return;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  uint32_t *row = bits + (uint64_t)r * stride;
+  const uint32_t n_units = stride / kPresUnitWords;
+  uint32_t carry = 0u;
+  for (uint32_t u0 = 0; u0 < n_units; u0 += kRankThreads) {
+    const uint32_t u = u0 + threadIdx.x;
+    uint32_t c = 0u;
+    if (u < n_units) {
+      const uint4 *p = reinterpret_cast<const uint4 *>(row + (uint64_t)u * kPresUnitWords);
+      const uint4 a = p[0], b = p[1];
+      c = __popc(a.y) + __popc(a.z) + __popc(a.w) + __popc(b.x) + __popc(b.y) + __popc(b.z) + __popc(b.w);
+    }
+    uint32_t incl = c;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const uint32_t v = __shfl_up_sync(0xFFFFFFFFu, incl, o);
+      if (lane >= o) incl += v;
+    }
+    if (lane == 31) s_warp[warp] = incl;
+    __syncthreads();
+    if (warp == 0) {
+      uint32_t t = s_warp[lane], ti = t;
+#pragma unroll
+      for (int o = 1; o < 32; o <<= 1) {
+        const uint32_t v = __shfl_up_sync(0xFFFFFFFFu, ti, o);
+        if (lane >= o) ti += v;
+      }
+      s_warp[lane] = ti - t;
+      if (lane == 31) s_warp[kRankThreads / 32] = ti;
+    }
+    __syncthreads();
+    if (u < n_units) row[(uint64_t)u * kPresUnitWords] = carry + s_warp[warp] + incl - c;
+    carry += s_warp[kRankThreads / 32];
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) totals[r] = carry;
 }
 
 // one warp per (512-doc slice, column): the exact maximum contribution inside the slice

@@ -66,7 +66,8 @@ struct ScanDev {
   uint32_t two_rounds;       // verification asks the lower-priority lists first, the higher-priority ones only for the survivors
   uint32_t part_lo, part_hi; // this launch scans items [n_items * part_lo / 256, n_items * part_hi / 256): 0..256 = all.  Sharded
                              // runs scan the rarest items first, exchange the per-query k-th keys, then scan the rest
-  unsigned long long *counters;  // [8]: 0 postings scanned, 3 items scanned, 4 postings verified, 5 items dropped by MaxScore
+  unsigned long long *counters;  // [8]: 0 postings scanned, 3 items scanned, 4 postings verified, 5 items dropped by MaxScore,
+                                 // sparse look-ups of the verification: 6 answered by a presence bitmap, 7 by lower_bound_interp
 };
 
 // largest unit-weight contribution of every unique term of the batch: a reduction over the term's resident scores.
@@ -360,8 +361,8 @@ __global__ void __launch_bounds__(kScanWarps * 32, 4) slg_scan_kernel(SegmentDev
   const uint32_t n_all = *sc.n_items;
   const uint32_t item_lo = (uint32_t)(((uint64_t)n_all * sc.part_lo) >> 8), n_items = (uint32_t)(((uint64_t)n_all * sc.part_hi) >> 8);
   uint32_t *work = sc.counter + (sc.part_lo ? 1 : 0);
-  const float inv_docs = 1.0f / (float)max(seg.doc_count, 1u);
-  unsigned long long n_scanned = 0, n_verified = 0, n_lookups = 0;
+  unsigned long long n_scanned = 0;
+  uint32_t n_lane_verified = 0, n_lane_bit_lookups = 0, n_lane_searches = 0;  // (per lane: a few 10^4 per launch)
   uint32_t n_dropped = 0, n_done = 0;
   WarpCand wc;
 
@@ -388,9 +389,8 @@ __global__ void __launch_bounds__(kScanWarps * 32, 4) slg_scan_kernel(SegmentDev
       // lane u < nt keeps term u of the query: what verify needs, handed round by shuffles
       uint64_t m_base = 0;      // first posting of the term's list
       uint64_t m_col = 0;       // column terms: element offset of the column
-      uint64_t m_bits = 0;      // sparse: word offset of the term's presence bitmap in seg.pres_bits, ~0 = none
-      uint32_t m_df = 0, m_kind = 0;  // kind: 0 absent / unscored, 1 sparse, 2 column
-      float m_w = 0.0f, m_ub = 0.0f, m_dens = 0.0f;
+      uint32_t m_df = 0, m_kind = 0;  // kind: 0 absent / unscored, 1 sparse, 2 column, 3 sparse with a presence bitmap (m_df = its row)
+      float m_w = 0.0f, m_ub = 0.0f;
       if (lane < (int)nt) {
         const QTerm q = qts[lane];
         if (q.flags & 1u) {
@@ -408,11 +408,10 @@ __global__ void __launch_bounds__(kScanWarps * 32, 4) slg_scan_kernel(SegmentDev
             m_kind = 1;
             m_base = q.base;
             m_df = __ldg(seg.term_df + q.term);
-            m_dens = (float)m_df * inv_docs;
-            m_bits = ~0ull;
-            if (seg.term_bits) {
-              const int32_t row = __ldg(seg.term_bits + q.term);
-              if (row >= 0) m_bits = (uint64_t)row * seg.bits_stride;
+            const int32_t row = seg.term_bits ? __ldg(seg.term_bits + q.term) : -1;
+            if (row >= 0) {
+              m_kind = 3;
+              m_df = (uint32_t)row;
             }
           }
         }
@@ -444,13 +443,13 @@ __global__ void __launch_bounds__(kScanWarps * 32, 4) slg_scan_kernel(SegmentDev
         qhead += n;
         nq -= n;
         alive = alive && __float_as_uint(v) >= cut;  // (the k-th score may have risen since the posting was queued)
-        n_verified += alive ? 1u : 0u;
+        n_lane_verified += alive ? 1u : 0u;
         // a filtered query asks the filter first: one bit, and at a selectivity of a few percent most docs are done here
         if (alive && pr.filter >= 0) alive = (__ldg(wb.filter_bits[pr.filter] + (doc >> 5)) >> (doc & 31)) & 1u;
         const bool must = MUST;
-        // ---- verify, cheapest evidence first: the column terms (one gather each), then the other sparse terms (a bit test,
-        // a search when the bit is set), dropping the doc as soon as  known contributions + bounds of the unknown ones  falls
-        // below the k-th score.  The exact score is the sum of the contributions in slot order.
+        // ---- verify, cheapest evidence first: the column terms (one gather each), then the other sparse terms (a presence
+        // bitmap look-up, or a search for a term without a bitmap), dropping the doc as soon as  known contributions + bounds
+        // of the unknown ones  falls below the k-th score.  The exact score is the sum of the contributions in slot order.
         const float thr_s = wc.thr == kThrInit ? 0.0f : __uint_as_float((uint32_t)(wc.thr >> 32)) * 0.99998f;
         float c[kWarpMaxTerms];
         float known = v, unknown = pr.others;  // (pr.others = the bounds of exactly the terms that can still add: columns + lower-priority sparse)
@@ -480,25 +479,34 @@ __global__ void __launch_bounds__(kScanWarps * 32, 4) slg_scan_kernel(SegmentDev
 #pragma unroll
         for (int u = 0; u < (int)kWarpMaxTerms; u++) {
           const uint32_t kind = __shfl_sync(0xFFFFFFFFu, m_kind, u);
-          if (kind != 1u || u == (int)t) continue;  // (uniform)
+          if (!(kind & 1u) || u == (int)t) continue;  // (uniform)
           const float ub = __shfl_sync(0xFFFFFFFFu, m_ub, u);
           const bool higher = !must && (ub > my_ub || (ub == my_ub && u < (int)t));  // a holder of higher priority offers the doc itself
           if (n_rounds == 2 && higher != (round == 1)) continue;  // (uniform)
           if (!__any_sync(0xFFFFFFFFu, alive)) break;
-          const uint64_t pb = __shfl_sync(0xFFFFFFFFu, m_base, u), bo = __shfl_sync(0xFFFFFFFFu, m_bits, u);
-          const uint32_t dfu = __shfl_sync(0xFFFFFFFFu, m_df, u);
-          const float w = __shfl_sync(0xFFFFFFFFu, m_w, u), dens = __shfl_sync(0xFFFFFFFFu, m_dens, u);
+          const uint64_t pb = __shfl_sync(0xFFFFFFFFu, m_base, u);
+          const uint32_t dfu = __shfl_sync(0xFFFFFFFFu, m_df, u);  // (kind 3: the bitmap row)
+          const float w = __shfl_sync(0xFFFFFFFFu, m_w, u);
           if (alive) {
-            n_lookups++;
-            const uint32_t *dp = seg.post_doc + pb;
-            // one bit per doc says whether the list holds it at all (one sector instead of a search: usually it does not)
-            bool held = true;
-            if (bo != ~0ull) held = (__ldg(seg.pres_bits + bo + (doc >> 5)) >> (doc & 31)) & 1u;
-            const uint32_t at = held ? lower_bound_interp(dp, dfu, doc, dens) : dfu;
-            if (at < dfu && __ldg(dp + at) == doc) {
-              if (higher) stand_back = true;
-              c[u] = __fmul_rn(__ldg(wb.scores + pb + at), w);
-              known += c[u];
+            bool held;
+            uint32_t at = 0u;
+            if (kind == 3u) {
+              // the term's presence bitmap: bit and list position from one sector, post_doc is not read
+              n_lane_bit_lookups++;
+              held = presence_lookup(seg, (uint64_t)dfu * seg.bits_stride, doc, at);
+            } else {
+              n_lane_searches++;
+              const uint32_t *dp = seg.post_doc + pb;
+              at = lower_bound_interp(dp, dfu, doc, (float)dfu * (1.0f / (float)max(seg.doc_count, 1u)));
+              held = at < dfu && __ldg(dp + at) == doc;
+            }
+            if (held) {
+              if (higher) {
+                stand_back = true;  // (the doc dies here: its contribution is not needed)
+              } else {
+                c[u] = __fmul_rn(__ldg(wb.scores + pb + at), w);
+                known += c[u];
+              }
             } else if (must) {
               stand_back = true;  // an AND query's doc must sit in every list
             }
@@ -569,16 +577,19 @@ __global__ void __launch_bounds__(kScanWarps * 32, 4) slg_scan_kernel(SegmentDev
     item = __shfl_sync(0xFFFFFFFFu, next_item, 0);
   }
   if (sc.counters) {
+    unsigned long long n_verified = n_lane_verified, n_bit_lookups = n_lane_bit_lookups, n_searches = n_lane_searches;
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
       n_verified += __shfl_xor_sync(0xFFFFFFFFu, n_verified, o);
-      n_lookups += __shfl_xor_sync(0xFFFFFFFFu, n_lookups, o);
+      n_bit_lookups += __shfl_xor_sync(0xFFFFFFFFu, n_bit_lookups, o);
+      n_searches += __shfl_xor_sync(0xFFFFFFFFu, n_searches, o);
     }
     if (lane == 0) {
       if (n_scanned) atomicAdd(sc.counters + 0, n_scanned);
       if (n_verified) atomicAdd(sc.counters + 4, n_verified);
       if (n_dropped) atomicAdd(sc.counters + 5, (unsigned long long)n_dropped);
-      if (n_lookups) atomicAdd(sc.counters + 6, n_lookups);
+      if (n_bit_lookups) atomicAdd(sc.counters + 6, n_bit_lookups);
+      if (n_searches) atomicAdd(sc.counters + 7, n_searches);
       if (n_done) atomicAdd(sc.counters + 3, (unsigned long long)n_done);
     }
   }

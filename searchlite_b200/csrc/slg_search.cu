@@ -928,6 +928,9 @@ int32_t slg_batch_fetch(slg_batch_t *bt, slg_hit_t *out_hits, uint32_t *out_coun
   ix->ctr.last_items = ic[3];
   ix->ctr.last_postings_verified = ic[4];
   ix->ctr.last_items_dropped = ic[5];
+  // SLG_SCAN_TRACE=1: where the flat scan's verification looked up the other sparse terms of a query
+  if (getenv("SLG_SCAN_TRACE"))
+    fprintf(stderr, "[slg scan] verified %llu, sparse look-ups answered by a presence bitmap %llu, by lower_bound_interp %llu\n", ic[4], ic[6], ic[7]);
   if (out_stats) {
     for (uint32_t q = 0; q < bt->Q; q++) {
       out_stats[q].scored_docs = sv[q * 4 + 0];

@@ -37,6 +37,7 @@
 #pragma once
 #include "slg_async.cuh"
 #include "slg_items_kernel.cuh"
+#include "slg_residency.cuh"
 
 namespace slg {
 
@@ -940,17 +941,19 @@ __device__ __forceinline__ float verify_doc(const SegmentDev &seg, const WarpBat
         const uint32_t term = __ldg(&qts[u].term);
         if (term < seg.n_terms) {
           const uint64_t base = __ldg(&qts[u].base);
-          const uint32_t *dp = seg.post_doc + base;
-          const uint32_t end = __ldg(seg.term_df + term);
-          // one bit per doc says whether the list holds it at all; a search only when it does
-          bool held = true;
-          if (seg.term_bits) {
-            const int32_t row = __ldg(seg.term_bits + term);
-            if (row >= 0) held = (__ldg(seg.pres_bits + (uint64_t)row * seg.bits_stride + (doc >> 5)) >> (doc & 31)) & 1u;
+          const int32_t row = seg.term_bits ? __ldg(seg.term_bits + term) : -1;
+          bool held;
+          uint32_t at = 0u;
+          if (row >= 0) {
+            held = presence_lookup(seg, (uint64_t)row * seg.bits_stride, doc, at);  // bit and list position from one sector
+          } else {
+            const uint32_t *dp = seg.post_doc + base;
+            const uint32_t end = __ldg(seg.term_df + term);
+            at = lower_bound_interp(dp, end, doc, (float)end / (float)max(seg.doc_count, 1u));
+            held = at < end && __ldg(dp + at) == doc;
           }
-          const uint32_t lo = held ? lower_bound_interp(dp, end, doc, (float)end / (float)max(seg.doc_count, 1u)) : end;
-          if (lo < end && __ldg(dp + lo) == doc) {
-            c = __ldg(wb.scores + base + lo);
+          if (held) {
+            c = __ldg(wb.scores + base + at);
             holders |= 1u << u;
           }
         }
