@@ -56,7 +56,11 @@ enum { SLG_TERM_SCORED = 1u };
 /* One "field:term" key of a query after search_segment's weight merge (api/reader.rs:2971-2983). */
 typedef struct {
   uint32_t term_id; /* ordinal of the key in the handle's term space; UINT32_MAX = absent */
-  float weight;     /* > 0; sum of group.boost*field.boost over duplicate keys */
+  float weight;     /* sum of group.boost*field.boost over duplicate keys.  A scored term's weight must be finite and
+                       >= 2^-100 (about 7.9e-31), else the batch fails with SLG_ERR_UNSUPPORTED: the kernels read a
+                       contribution of +0 as "the doc lacks the term" and never return a doc scored 0, while the reference
+                       keeps one.  From 2^-100 up, a posting's contribution stays above 2^-133 for any k1 >= 0, b in [0, 1]
+                       and doc less than 2^32 times longer than the average */
   uint32_t leaf;    /* ScorePlan leaf (Sum-of-leaves plan; list terms in leaf order) */
   uint32_t group;   /* matcher term group */
   uint32_t flags;   /* SLG_TERM_SCORED if it contributes to the score */

@@ -250,7 +250,12 @@ static __global__ void __launch_bounds__(128) slg_scan_pairs_kernel(SegmentDev s
           p.base = q.base;
           p.df = seg.term_df[sc.ut_term[q.uterm]];
           p.w = q.weight;
-          p.others = total_ub - ub[t];  // every other term must add its share
+          // every other term must add its share.  A direct sum: total_ub - ub[t] would round the other bounds to a multiple
+          // of ulp(total_ub), far off when the driver is heavily boosted
+          float o = 0.0f;
+          for (uint32_t u = 0; u < kWarpMaxTerms; u++)
+            if (u != t) o += ub[u];
+          p.others = o;
           p.ne_prefix = total_ub;       // below the k-th score: no doc of this query can enter the top k
         }
       } else if ((q.flags & 5u) == 1u && q.term < seg.n_terms) {
@@ -452,7 +457,12 @@ __global__ void __launch_bounds__(kScanWarps * 32, 4) slg_scan_kernel(SegmentDev
         // of the unknown ones  falls below the k-th score.  The exact score is the sum of the contributions in slot order.
         const float thr_s = wc.thr == kThrInit ? 0.0f : __uint_as_float((uint32_t)(wc.thr >> 32)) * 0.99998f;
         float c[kWarpMaxTerms];
-        float known = v, unknown = pr.others;  // (pr.others = the bounds of exactly the terms that can still add: columns + lower-priority sparse)
+        // unknown starts at pr.others (the bounds of exactly the terms that can still add: columns + lower-priority sparse)
+        // and loses each bound once its term is looked up.  pr.others is a rounded sum and every subtraction rounds again:
+        // up to 8 ulp(pr.others) in all, an absolute error that the relative slacks below do not cover when a boosted term's
+        // bound dwarfs the others (after a column bound of 3e5 is taken off, a bound of 1.1 would be left as 1.09375).
+        // 2^-19 * pr.others (>= 16 ulp) covers it
+        float known = v, unknown = __fadd_rn(pr.others, __fmul_rn(pr.others, 0x1p-19f));
 #pragma unroll
         for (int u = 0; u < (int)kWarpMaxTerms; u++) {
           c[u] = 0.0f;

@@ -158,8 +158,8 @@ int32_t slg_batch_prepare(slg_index_t *ix, const slg_query_t *queries, uint32_t 
       const slg_term_t &tm = q.terms[t];
       if (tm.term_id == 0xFFFFFFFFu || tm.term_id >= n_terms_space) continue;  // seg.postings(key) == None
       bool scored = tm.flags & SLG_TERM_SCORED;
-      if (scored && !(tm.weight > 0.0f && std::isfinite(tm.weight)))
-        return fail(ix, SLG_ERR_UNSUPPORTED, "query %u term %u: weight must be finite and > 0", qi, t);
+      if (scored && !(tm.weight >= 0x1p-100f && std::isfinite(tm.weight)))  // (below: a contribution may round to +0, include/searchlite_gpu.h)
+        return fail(ix, SLG_ERR_UNSUPPORTED, "query %u term %u: weight must be finite and >= 2^-100", qi, t);
       if (q.n_groups && tm.group >= q.n_groups) return fail(ix, SLG_ERR_INVALID, "query %u term %u: group out of range", qi, t);
       if (scored && q.n_plan_nodes && tm.leaf >= q.leaf_count)
         return fail(ix, SLG_ERR_INVALID, "query %u term %u: leaf %u but the plan has %u leaves", qi, t, tm.leaf, q.leaf_count);  // wand.rs:489-494
