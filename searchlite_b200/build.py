@@ -13,7 +13,7 @@ LIB_PATH = os.path.join(LIB_DIR, "libsearchlite_gpu.so")
 SOURCES = ["slg_engine.cu", "slg_search.cu", "slg_rerank.cu", "slg_launch_tiles.cu", "slg_launch_warp.cu", "slg_launch_items.cu"]
 HEADERS = ["slg_kernels.cuh", "slg_phrase.cuh", "slg_segfiles.h", "slg_warp_kernel.cuh", "slg_items_kernel.cuh", "slg_stream_kernel.cuh", "slg_scan_kernel.cuh",
            "slg_residency.cuh", "slg_async.cuh",
-           "slg_host.h", "slg_launch.h", "slg_filter.cuh", "slg_postimage.cuh", "slg_rerank.cuh",
+           "slg_host.h", "slg_dispatch.h", "slg_launch.h", "slg_filter.cuh", "slg_postimage.cuh", "slg_rerank.cuh",
            os.path.join("..", "..", "include", "searchlite_gpu.h")]
 
 NVCC_FLAGS = [

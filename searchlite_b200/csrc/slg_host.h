@@ -18,6 +18,7 @@
 
 #include <cuda_runtime.h>
 
+#include "slg_dispatch.h"
 #include "slg_launch.h"
 
 namespace slg {
@@ -300,11 +301,8 @@ struct slg_batch {
   uint32_t items_cap = 0;
   unsigned char *results = nullptr;   // per segment: hits [Q][k], counts [Q], vector scores [Q][k] (after a rerank); then the merged block (S > 1)
   size_t result_stride = 0;           // bytes of one such block
-  bool staged = false;                // the (doc, score) stream form of the warp kernel applies
   uint32_t max_terms = 0;
-  bool use_warp = false, can_items = false, canonical = false;
-  bool and_scan = false;              // every query is Bool{must: one term per group}: the posting scan drives from the rarest list
-  bool big_k = false;                 // k > 32 on the flat posting scan: candidate pools
+  slg::Selection sel;                 // which kernels the batch may take (slg_dispatch.h)
   unsigned long long *pool_keys = nullptr;
   uint32_t *pool_count = nullptr, *pool_lock = nullptr;
   uint32_t pool_cap = 0;

@@ -4,6 +4,10 @@
 // Mirrors IndexReader::search_segment (searchlite-core/src/api/reader.rs:2908-3128) and
 // execute_top_k_with_stats_and_mode_internal (src/query/wand.rs:398-456) for Q queries at once, and
 // hits.sort_by(SortKey) (api/reader.rs:2777).  There is no CPU fallback: every search runs the CUDA kernels or fails.
+#include <functional>
+#include <tuple>
+#include <type_traits>
+
 #include "slg_host.h"
 #include "slg_residency.cuh"
 
@@ -37,6 +41,12 @@ struct TermSet {
     }
   }
 };
+
+// CTAs per SM that `smem` bytes of dynamic shared memory allow, at most `cap` and at most the ctas_per_sm option
+uint32_t ctas_for_smem(const slg_index *ix, size_t smem, uint32_t cap) {
+  const uint32_t n = std::min((uint32_t)std::max<size_t>(1, (ix->smem_optin + 1024) / (smem + 1024)), cap);
+  return ix->ctas_per_sm ? std::min(n, ix->ctas_per_sm) : n;
+}
 
 int32_t select_smem(slg_index *ix, uint32_t tile_docs, uint32_t cap, bool matcher, size_t *out, uint32_t planes = 1) {
   size_t smem = (size_t)tile_docs * 4 * planes + (size_t)cap * 8 + (matcher ? tile_docs : 0);
@@ -103,10 +113,10 @@ int32_t slg_batch_prepare(slg_index_t *ix, const slg_query_t *queries, uint32_t 
   qt_g.reserve(t_expect);
   qt_f.reserve(t_expect);
   qt_leaf.reserve(t_expect);
-  bool matcher = false;
+  BatchFacts facts;  // what the kernel selection (slg_dispatch.h) needs to know
   // AND batches: every query is Bool{must:[t1, t2, ..]} — one scored term per group, every group a MUST, nothing else.  The
   // posting scan then walks only the query's RAREST list and asks the other lists whether they hold the doc
-  bool all_must = true;
+  facts.all_must = true;
   for (uint32_t qi = 0; qi < n_queries; qi++) {
     const slg_query_t &q = queries[qi];
     if (q.n_terms && !q.terms) return fail(ix, SLG_ERR_INVALID, "query %u has no terms pointer", qi);
@@ -180,13 +190,13 @@ int32_t slg_batch_prepare(slg_index_t *ix, const slg_query_t *queries, uint32_t 
         pure = (q.terms[t].flags & SLG_TERM_SCORED) && !((seen_groups >> q.terms[t].group) & 1u);
         seen_groups |= 1u << q.terms[t].group;
       }
-      all_must = all_must && pure;
+      facts.all_must = facts.all_must && pure;
     }
     if (kept > SLG_MAX_QUERY_TERMS) return fail(ix, SLG_ERR_UNSUPPORTED, "query %u has %u terms; the maximum is %u", qi, kept, SLG_MAX_QUERY_TERMS);
     q_off[qi + 1] = q_off[qi] + kept;
     bt->max_terms = std::max(bt->max_terms, kept);
     if (need_mask) {
-      matcher = true;
+      facts.matcher = true;
       if (q.n_groups == 0) {  // non-scored terms without groups: plain OR over group 0
         q_should[qi] = 1;
         q_min[qi] = 1;
@@ -225,35 +235,24 @@ int32_t slg_batch_prepare(slg_index_t *ix, const slg_query_t *queries, uint32_t 
     }
     bt->n_cursor_segs = S;
   }
-  bt->matcher = matcher;
+  bt->matcher = facts.matcher;
   bt->U = (uint32_t)ut.size();
   bt->T = (uint32_t)qt_u.size();
 
   // ---- kernel selection ----
-  // items kernel (posting-driven; the automatic choice): plain OR queries, k <= 32, <= 8 terms per query, resident
-  // scores, no plan.  Per-query statistics are counted by the warp kernel, on the same (canonical) term layout.
-  const bool small = k <= kWarpMaxK && bt->max_terms <= kWarpMaxTerms;
-  bool all_scores = ix->staging;
-  for (auto &s : ix->segs) all_scores = all_scores && (s->post_score.p != nullptr || s->n_blocks == 0);
-  // (AND batches ride the posting scan; without it — scan_kernels 0, statistics — they are ordinary matcher batches)
-  const bool and_scan = matcher && all_must && ix->scan_kernels && ix->stream_kernels && !bt->has_cursor;
-  bt->and_scan = and_scan;
-  const bool items_ok = small && (!matcher || and_scan) && all_scores && !bt->has_plan && ix->sub_docs <= 4096;
-  bt->can_items = items_ok && (ix->kernel_choice == 0 || ix->kernel_choice == 3);
-  // k up to SLG_MAX_K on the flat posting scan: candidate pools + radix select instead of the warp's sorted top-k
-  bt->big_k = k > kWarpMaxK && bt->max_terms <= kWarpMaxTerms && (!matcher || and_scan) && all_scores && !bt->has_plan && ix->scan_kernels && ix->stream_kernels &&
-              (ix->kernel_choice == 0 || ix->kernel_choice == 3);
-  if (bt->big_k) bt->can_items = true;
-  if (ix->kernel_choice == 3 && !items_ok && !bt->big_k)
-    return fail(ix, SLG_ERR_UNSUPPORTED,
-                "the items kernel handles plain OR queries without a ScorePlan, k <= %u, <= %u terms per query, resident scores, sub_docs <= 4096",
-                kWarpMaxK, kWarpMaxTerms);
-
-  bt->canonical = bt->can_items;
-  bt->use_warp = bt->can_items || ix->kernel_choice == 2 || (ix->kernel_choice == 0 && small);
-  if (bt->use_warp && !small && !bt->big_k)
-    return fail(ix, SLG_ERR_UNSUPPORTED, "the warp kernel handles k <= %u and <= %u terms per query", kWarpMaxK, kWarpMaxTerms);
-  bt->staged = all_scores && !matcher && bt->U > 0;
+  facts.kernel_choice = ix->kernel_choice;
+  facts.small_k = k <= kWarpMaxK;
+  facts.few_terms = bt->max_terms <= kWarpMaxTerms;
+  facts.has_cursor = bt->has_cursor;
+  facts.has_plan = bt->has_plan;
+  facts.all_scores = ix->staging;
+  for (auto &s : ix->segs) facts.all_scores = facts.all_scores && (s->post_score.p != nullptr || s->n_blocks == 0);
+  facts.sub_docs_ok = ix->sub_docs <= 4096;
+  facts.scan_kernels = ix->scan_kernels;
+  facts.stream_kernels = ix->stream_kernels;
+  facts.has_terms = bt->U > 0;
+  if (const char *why = select_kernels(facts, bt->sel)) return fail(ix, SLG_ERR_UNSUPPORTED, why, kWarpMaxK, kWarpMaxTerms);
+  const Selection &sel = bt->sel;
 
   // processing order inside a tile: most expensive queries first
   std::vector<uint32_t> order(n_queries);
@@ -261,12 +260,12 @@ int32_t slg_batch_prepare(slg_index_t *ix, const slg_query_t *queries, uint32_t 
   std::stable_sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b2) { return q_cost[a] > q_cost[b2]; });
 
   // ---- geometry ----
-  bt->plan_docs = bt->use_warp ? ix->sub_docs : ix->tile_docs;
+  bt->plan_docs = sel.warp_tables ? ix->sub_docs : ix->tile_docs;
   if (bt->has_plan) {
     // one accumulator plane per leaf: shrink the doc tile so that the planes together stay near the configured tile
     uint32_t planes = 1;
     while (planes < bt->max_leaves) planes <<= 1;
-    bt->plan_docs = bt->use_warp ? std::max(512u, (ix->sub_docs / planes) & ~127u) : std::max(1024u, (ix->tile_docs / planes) & ~1023u);
+    bt->plan_docs = sel.warp_tables ? std::max(512u, (ix->sub_docs / planes) & ~127u) : std::max(1024u, (ix->tile_docs / planes) & ~1023u);
   }
   uint32_t max_tiles = 1;
   for (auto &s : ix->segs) max_tiles = std::max(max_tiles, (s->doc_count + bt->plan_docs - 1) / bt->plan_docs);
@@ -275,59 +274,62 @@ int32_t slg_batch_prepare(slg_index_t *ix, const slg_query_t *queries, uint32_t 
 
   // ---- packed inputs: one host-to-device copy out of pinned memory ----
   size_t pos = 0;
-  auto place = [&](size_t bytes) {
-    size_t o = pos;
+  std::vector<std::tuple<size_t, const void *, size_t>> inputs;  // (offset, source, bytes), copied once pinned memory is held
+  auto place = [&](size_t &off, const void *src, size_t bytes) {
+    off = pos;
     pos = align_up(pos + std::max<size_t>(bytes, 4), 256);
-    return o;
+    inputs.emplace_back(off, src, bytes);
   };
-  bt->off_ut_term = place((size_t)bt->U * 4);
-  bt->off_q_term_off = place((size_t)(n_queries + 1) * 4);
-  bt->off_qt_uterm = place((size_t)bt->T * 4);
-  bt->off_qt_weight = place((size_t)bt->T * 4);
-  bt->off_qt_group = place(bt->T);
-  bt->off_qt_flags = place(bt->T);
-  bt->off_q_order = place((size_t)n_queries * 4);
-  bt->off_q_must = place(n_queries);
-  bt->off_q_not = place(n_queries);
-  bt->off_q_should = place(n_queries);
-  bt->off_q_min = place(n_queries);
-  bt->off_q_filter = place((size_t)n_queries * 4);
+  place(bt->off_ut_term, ut.data(), (size_t)bt->U * 4);
+  place(bt->off_q_term_off, q_off.data(), (size_t)(n_queries + 1) * 4);
+  place(bt->off_qt_uterm, qt_u.data(), (size_t)bt->T * 4);
+  place(bt->off_qt_weight, qt_w.data(), (size_t)bt->T * 4);
+  place(bt->off_qt_group, qt_g.data(), bt->T);
+  place(bt->off_qt_flags, qt_f.data(), bt->T);
+  place(bt->off_q_order, order.data(), (size_t)n_queries * 4);
+  place(bt->off_q_must, q_must.data(), n_queries);
+  place(bt->off_q_not, q_not.data(), n_queries);
+  place(bt->off_q_should, q_should.data(), n_queries);
+  place(bt->off_q_min, q_min.data(), n_queries);
+  place(bt->off_q_filter, q_filter.data(), (size_t)n_queries * 4);
   if (bt->has_plan) {
-    bt->off_qt_leaf = place(bt->T);
-    bt->off_q_leaves = place(n_queries);
-    bt->off_q_plan_off = place((size_t)(n_queries + 1) * 4);
-    bt->off_plan_nodes = place(plan_nodes.size() * sizeof(PlanNodeDev));
+    place(bt->off_qt_leaf, qt_leaf.data(), bt->T);
+    place(bt->off_q_leaves, q_leaves.data(), n_queries);
+    place(bt->off_q_plan_off, q_plan_off.data(), (size_t)(n_queries + 1) * 4);
+    place(bt->off_plan_nodes, plan_nodes.data(), plan_nodes.size() * sizeof(PlanNodeDev));
   }
-  if (bt->has_cursor) bt->off_cursor_bounds = place(bounds.size() * 8);
+  if (bt->has_cursor) place(bt->off_cursor_bounds, bounds.data(), bounds.size() * 8);
   bt->pack_bytes = pos;
 
-  // ---- the slab ----
+  // ---- the slab: every section is named once; its pointer is bound once the slab exists (absent: nullptr) ----
   size_t dpos = 0;
-  auto carve = [&](size_t bytes) {
-    size_t o = dpos;
+  std::vector<std::function<void(unsigned char *)>> bind;
+  auto carve = [&](auto *&ptr, bool want, size_t bytes) {
+    ptr = nullptr;
+    if (!want) return;
+    const size_t o = dpos;
     dpos = align_up(dpos + std::max<size_t>(bytes, 16), 256);
-    return o;
+    bind.push_back([&ptr, o](unsigned char *base) { ptr = reinterpret_cast<std::remove_reference_t<decltype(ptr)>>(base + o); });
   };
-  const size_t o_pack = carve(bt->pack_bytes);
-  const size_t o_rng = carve((size_t)std::max(bt->U, 1u) * (max_tiles + 1) * 4);
-  const size_t o_ub = (exec != SLG_EXEC_BM25 || bt->can_items) ? carve((size_t)std::max(bt->U, 1u) * max_tiles * 4) : 0;
+  carve(bt->d_pack, true, bt->pack_bytes);
+  carve(bt->ut_rng, true, (size_t)std::max(bt->U, 1u) * (max_tiles + 1) * 4);
+  carve(bt->ut_tile_ub, exec != SLG_EXEC_BM25 || sel.canonical, (size_t)std::max(bt->U, 1u) * max_tiles * 4);
   // state block, reset per segment: thr_key [Q] u64 | topk_count [Q] | lock [Q] | work_counter [64] | n_items [2]
   uint32_t kp = 1;
   while (kp < k) kp <<= 1;
-  bt->pool_cap = bt->big_k ? 2 * kp : 0;
-  const size_t state_words = (size_t)n_queries * 2 + 64 + 2 + (bt->big_k ? (size_t)n_queries * 4 : 0);
-  const size_t o_thr = carve((size_t)n_queries * 8 + state_words * 4);
-  const size_t o_topk = carve((size_t)n_queries * k * 8);
-  const size_t o_pools = bt->big_k ? carve((size_t)n_queries * 2 * bt->pool_cap * 8) : 0;
-  const size_t o_stats = carve((size_t)n_queries * 5 * 8 + 64);  // [Q][4] counters, [Q] accepted docs, then the items counters [4]
-  const size_t o_saw = bt->has_cursor ? carve((size_t)n_queries * 4) : 0;
-  const size_t o_qterms = bt->use_warp ? carve((size_t)n_queries * kWarpMaxTerms * sizeof(QTerm)) : 0;
-  const size_t o_qheads = bt->use_warp ? carve((size_t)n_queries * sizeof(QHead)) : 0;
-  const bool want_items = bt->can_items && exec != SLG_EXEC_BM25;
+  bt->pool_cap = sel.pools ? 2 * kp : 0;
+  const size_t state_words = (size_t)n_queries * 2 + 64 + 2 + (sel.pools ? (size_t)n_queries * 4 : 0);
+  carve(bt->thr_key, true, (size_t)n_queries * 8 + state_words * 4);
+  carve(bt->topk_keys, true, (size_t)n_queries * k * 8);
+  carve(bt->pool_keys, sel.pools, (size_t)n_queries * 2 * bt->pool_cap * 8);
+  carve(bt->stats, true, (size_t)n_queries * 5 * 8 + 64);  // [Q][4] counters, [Q] accepted docs, then the items counters [4]
+  carve(bt->cursor_saw, bt->has_cursor, (size_t)n_queries * 4);
+  carve(bt->qterms, sel.warp_tables, (size_t)n_queries * kWarpMaxTerms * sizeof(QTerm));
+  carve(bt->qheads, sel.warp_tables, (size_t)n_queries * sizeof(QHead));
+  const bool want_items = sel.canonical && exec != SLG_EXEC_BM25;
   bt->items_cap = want_items ? max_groups * n_queries : 0;
   bt->done_bytes = want_items ? (size_t)max_groups * n_queries : 0;
-  const size_t o_items = want_items ? carve((size_t)bt->items_cap * sizeof(uint2)) : 0;
-  const bool want_stream = bt->can_items && ix->stream_kernels;
+  carve(bt->items, want_items, (size_t)bt->items_cap * sizeof(uint2));
   for (auto &s : ix->segs) bt->max_cols = std::max(bt->max_cols, s->n_cols);
   // postings per scan item: 4096 on a 10 M-doc segment (fewer, longer items: less per-item work), smaller on small
   // segments — the shards of a multi-GPU run — where 4096 leaves too few items to balance 4736 warps
@@ -338,62 +340,40 @@ int32_t slg_batch_prepare(slg_index_t *ix, const slg_query_t *queries, uint32_t 
     bt->scan_chunk = ix->scan_chunk ? ix->scan_chunk : (max_docs >= 4000000u ? 4096u : max_docs >= 2000000u ? 2048u : 1024u);
   }
   // flat posting scan: item capacity = the largest segment's sum over scanned term instances of ceil(df / scan_chunk)
-  if (bt->can_items) {
+  if (sel.canonical) {
     for (auto &sg : ix->segs) {
       uint64_t n = 0;
       for (size_t i = 0; i < qt_u.size(); i++) {
         const uint32_t term = ut[qt_u[i]];
         if (term >= sg->n_terms || !qt_f[i]) continue;
-        if (!bt->and_scan && !sg->h_term_col.empty() && sg->h_term_col[term] >= 0) continue;  // (an AND batch may scan any of its terms)
+        if (!sel.and_scan && !sg->h_term_col.empty() && sg->h_term_col[term] >= 0) continue;  // (an AND batch may scan any of its terms)
         n += (sg->h_df[term] + bt->scan_chunk - 1) / bt->scan_chunk;
       }
       bt->scan_items_cap = (uint32_t)std::max<uint64_t>(bt->scan_items_cap, std::min<uint64_t>(n, 0xFFFFFFF0ull));
     }
   }
-  const bool want_scan = bt->can_items;
-  const size_t o_utmax = want_scan ? carve((size_t)std::max(bt->U, 1u) * 4) : 0;
-  const size_t o_pairs = want_scan ? carve((size_t)n_queries * kWarpMaxTerms * sizeof(ScanPair)) : 0;
-  const size_t o_order = want_scan ? carve((size_t)n_queries * kWarpMaxTerms * 4) : 0;
-  const size_t o_istart = want_scan ? carve(((size_t)n_queries * kWarpMaxTerms + 1) * 4) : 0;
-  const size_t o_sitems = want_scan ? carve((size_t)std::max(bt->scan_items_cap, 1u) * 4) : 0;
-  const size_t o_colq = want_stream ? carve((size_t)n_queries * sizeof(ColQ)) : 0;
-  const size_t o_ucol = want_stream ? carve((size_t)(bt->max_cols + 1) * 4) : 0;
-  const size_t o_colslot = want_stream ? carve((size_t)(bt->max_cols + 1) * 4) : 0;
-  const size_t o_done = want_items ? carve(bt->done_bytes) : 0;
+  carve(bt->ut_max, sel.canonical, (size_t)std::max(bt->U, 1u) * 4);
+  carve(bt->scan_pairs, sel.canonical, (size_t)n_queries * kWarpMaxTerms * sizeof(ScanPair));
+  carve(bt->scan_order, sel.canonical, (size_t)n_queries * kWarpMaxTerms * 4);
+  carve(bt->scan_item_start, sel.canonical, ((size_t)n_queries * kWarpMaxTerms + 1) * 4);
+  carve(bt->scan_items, sel.canonical, (size_t)std::max(bt->scan_items_cap, 1u) * 4);
+  carve(bt->colq, sel.colq, (size_t)n_queries * sizeof(ColQ));
+  carve(bt->ucol, sel.colq, (size_t)(bt->max_cols + 1) * 4);
+  carve(bt->col_slot, sel.colq, (size_t)(bt->max_cols + 1) * 4);
+  carve(bt->done, want_items, bt->done_bytes);
   bt->result_stride = align_up((size_t)n_queries * k * sizeof(HitDev) + (size_t)n_queries * 4 + (size_t)n_queries * k * 4, 256);  // hits | counts | vector scores
-  const size_t o_results = carve(bt->result_stride * (S + (S > 1 ? 1 : 0)));
+  carve(bt->results, true, bt->result_stride * (S + (S > 1 ? 1 : 0)));
   SLG_CUDA(ix, bt->slab.alloc(dpos));
-  unsigned char *base = bt->slab.as<unsigned char>();
-  bt->d_pack = base + o_pack;
-  bt->ut_rng = reinterpret_cast<uint32_t *>(base + o_rng);
-  bt->ut_tile_ub = (exec != SLG_EXEC_BM25 || bt->can_items) ? reinterpret_cast<float *>(base + o_ub) : nullptr;
-  bt->thr_key = reinterpret_cast<unsigned long long *>(base + o_thr);
-  bt->state = base + o_thr + (size_t)n_queries * 8;
+  for (auto &b : bind) b(bt->slab.as<unsigned char>());
+  bt->state = reinterpret_cast<unsigned char *>(bt->thr_key) + (size_t)n_queries * 8;
   bt->state_bytes = state_words * 4;
   bt->topk_count = reinterpret_cast<uint32_t *>(bt->state);
   bt->lock = bt->topk_count + n_queries;
   bt->work_counter = bt->lock + n_queries;
   bt->n_items = bt->work_counter + 64;
-  bt->pool_count = bt->big_k ? bt->n_items + 2 : nullptr;
-  bt->pool_lock = bt->big_k ? bt->pool_count + (size_t)n_queries * 2 : nullptr;
-  bt->pool_keys = bt->big_k ? reinterpret_cast<unsigned long long *>(base + o_pools) : nullptr;
-  bt->topk_keys = reinterpret_cast<unsigned long long *>(base + o_topk);
-  bt->stats = reinterpret_cast<unsigned long long *>(base + o_stats);
+  bt->pool_count = sel.pools ? bt->n_items + 2 : nullptr;
+  bt->pool_lock = sel.pools ? bt->pool_count + (size_t)n_queries * 2 : nullptr;
   bt->item_counters = bt->stats + (size_t)n_queries * 5;
-  bt->cursor_saw = bt->has_cursor ? reinterpret_cast<uint32_t *>(base + o_saw) : nullptr;
-  bt->qterms = bt->use_warp ? reinterpret_cast<QTerm *>(base + o_qterms) : nullptr;
-  bt->qheads = bt->use_warp ? reinterpret_cast<QHead *>(base + o_qheads) : nullptr;
-  bt->items = want_items ? reinterpret_cast<uint2 *>(base + o_items) : nullptr;
-  bt->done = want_items ? base + o_done : nullptr;
-  bt->ut_max = want_scan ? reinterpret_cast<float *>(base + o_utmax) : nullptr;
-  bt->scan_pairs = want_scan ? reinterpret_cast<ScanPair *>(base + o_pairs) : nullptr;
-  bt->scan_order = want_scan ? reinterpret_cast<uint32_t *>(base + o_order) : nullptr;
-  bt->scan_item_start = want_scan ? reinterpret_cast<uint32_t *>(base + o_istart) : nullptr;
-  bt->scan_items = want_scan ? reinterpret_cast<uint32_t *>(base + o_sitems) : nullptr;
-  bt->colq = want_stream ? reinterpret_cast<ColQ *>(base + o_colq) : nullptr;
-  bt->ucol = want_stream ? reinterpret_cast<uint32_t *>(base + o_ucol) : nullptr;
-  bt->col_slot = want_stream ? reinterpret_cast<uint32_t *>(base + o_colslot) : nullptr;
-  bt->results = base + o_results;
 
   // ---- pinned staging: [pack | results | per-query stats + items counters] ----
   bt->pinned_result_off = align_up(bt->pack_bytes, 256);
@@ -406,28 +386,8 @@ int32_t slg_batch_prepare(slg_index_t *ix, const slg_query_t *queries, uint32_t 
     SLG_CUDA(ix, cudaMallocHost(&bt->pinned, bt->pinned_bytes));
   }
   unsigned char *hp = static_cast<unsigned char *>(bt->pinned);
-  auto put = [&](size_t off, const void *src, size_t bytes) {
+  for (const auto &[off, src, bytes] : inputs)
     if (bytes) std::memcpy(hp + off, src, bytes);
-  };
-  put(bt->off_ut_term, ut.data(), (size_t)bt->U * 4);
-  put(bt->off_q_term_off, q_off.data(), (size_t)(n_queries + 1) * 4);
-  put(bt->off_qt_uterm, qt_u.data(), (size_t)bt->T * 4);
-  put(bt->off_qt_weight, qt_w.data(), (size_t)bt->T * 4);
-  put(bt->off_qt_group, qt_g.data(), bt->T);
-  put(bt->off_qt_flags, qt_f.data(), bt->T);
-  put(bt->off_q_order, order.data(), (size_t)n_queries * 4);
-  put(bt->off_q_must, q_must.data(), n_queries);
-  put(bt->off_q_not, q_not.data(), n_queries);
-  put(bt->off_q_should, q_should.data(), n_queries);
-  put(bt->off_q_min, q_min.data(), n_queries);
-  put(bt->off_q_filter, q_filter.data(), (size_t)n_queries * 4);
-  if (bt->has_plan) {
-    put(bt->off_qt_leaf, qt_leaf.data(), bt->T);
-    put(bt->off_q_leaves, q_leaves.data(), n_queries);
-    put(bt->off_q_plan_off, q_plan_off.data(), (size_t)(n_queries + 1) * 4);
-    put(bt->off_plan_nodes, plan_nodes.data(), plan_nodes.size() * sizeof(PlanNodeDev));
-  }
-  if (bt->has_cursor) put(bt->off_cursor_bounds, bounds.data(), bounds.size() * 8);
   SLG_CUDA(ix, cudaMemcpyAsync(bt->d_pack, hp, bt->pack_bytes, cudaMemcpyHostToDevice, ix->stream));
   ix->ctr.last_h2d_bytes = bt->pack_bytes;
   *out = bt.release();
@@ -438,44 +398,21 @@ int32_t slg_batch_prepare(slg_index_t *ix, const slg_query_t *queries, uint32_t 
 
 namespace {
 
-// everything of one run up to (seeds_only) or including the sweep; see the schedule in slg_batch_run
-int32_t run_batch(slg_batch *bt, bool do_seeds, bool do_sweep) {
-  slg_index *ix = bt->ix;
-  cudaStream_t st = ix->stream;
-  const bool prune = bt->exec != SLG_EXEC_BM25;
-  const uint32_t Q = bt->Q, k = bt->k;
-  const bool run_items = bt->can_items && !bt->want_stats && !(bt->big_k && (!ix->scan_kernels || (ix->strict_accumulate && bt->exec == SLG_EXEC_BM25)));
-  // flat posting scan + column pass: the automatic choice; scan_kernels 0 keeps the sub-tile kernels (stream / items)
-  const bool run_scan = run_items && ix->scan_kernels && bt->colq != nullptr && !(ix->strict_accumulate && !prune);
-  if (bt->and_scan && !run_scan && run_items)
-    return fail(ix, SLG_ERR_UNSUPPORTED, "an AND batch prepared for the posting scan cannot run on the sub-tile kernels (strict_accumulate)");
-  const bool two_step = !(do_seeds && do_sweep);
-  if (two_step && (ix->segs.size() != 1 || !run_items || (!prune && !run_scan)))
-    return fail(ix, SLG_ERR_UNSUPPORTED, "the two-step run (first part, threshold exchange, rest) needs one segment per handle and the posting scan or the pruned items kernel");
-  unsigned char *dp = bt->d_pack;
-  size_t smem = 0;
-  const bool run_scan_pre = bt->can_items && !bt->want_stats && ix->scan_kernels && bt->colq != nullptr && !(ix->strict_accumulate && !prune);
-  const bool warp_path = bt->use_warp && !(bt->big_k && !run_scan_pre);  // k > 32 without the scan: the CTA-per-item kernel
-  if (!warp_path) {
-    int32_t rc = bt->has_plan ? select_smem(ix, bt->plan_docs, bt->cap, bt->matcher, &smem, bt->max_leaves)
-                              : select_smem(ix, ix->tile_docs, bt->cap, bt->matcher, &smem);
-    if (rc) return rc;
-  }
-  uint32_t per_sm = (uint32_t)std::max<size_t>(1, (ix->smem_optin + 1024) / (smem + 1024));
-  per_sm = std::min(per_sm, 8u);
-  if (ix->ctas_per_sm) per_sm = std::min(per_sm, ix->ctas_per_sm);
-  if (do_seeds) {
-    SLG_CUDA(ix, cudaEventRecord(ix->ev[0], st));
-    SLG_CUDA(ix, cudaMemsetAsync(bt->stats, 0, (size_t)Q * 40 + 64, st));
-    if (bt->has_cursor) {
-      if (bt->n_cursor_segs != ix->segs.size()) return fail(ix, SLG_ERR_INVALID, "a segment was loaded after the batch with cursors was prepared");
-      SLG_CUDA(ix, cudaMemsetAsync(bt->cursor_saw, 0, (size_t)Q * 4, st));
-    }
-  }
-  uint32_t si = 0;
-  for (auto &sp : ix->segs) {
-    Segment *s = sp.get();
-    BatchDev bd{};
+// one segment's part of a run: the views of the batch that its kernels read, and one function per scoring path
+struct SegmentRun {
+  slg_batch *bt;
+  slg_index *ix;
+  cudaStream_t st;
+  bool prune;         // WAND / BMW
+  Segment *s;
+  BatchDev bd{};      // the plan kernels, the CTA-per-item kernel and the finalize
+  WarpBatchDev wb{};  // the warp-per-item, items and scan kernels (batches with warp tables)
+  ItemsDev it{};
+  size_t wsmem = 0;   // shared memory and grid of the warp-per-item and items kernels
+  int wgrid = 1;
+
+  void batch_view(uint32_t si) {
+    const unsigned char *dp = bt->d_pack;
     bd.ut_term = reinterpret_cast<const uint32_t *>(dp + bt->off_ut_term);
     bd.ut_rng = bt->ut_rng;
     bd.ut_tile_ub = bt->ut_tile_ub;
@@ -499,269 +436,329 @@ int32_t run_batch(slg_batch *bt, bool do_seeds, bool do_sweep) {
     }
     bd.max_leaves = bt->max_leaves;
     if (bt->has_cursor) {
-      bd.q_cursor = reinterpret_cast<const unsigned long long *>(dp + bt->off_cursor_bounds) + (size_t)si * Q;
+      bd.q_cursor = reinterpret_cast<const unsigned long long *>(dp + bt->off_cursor_bounds) + (size_t)si * bt->Q;
       bd.q_saw = bt->cursor_saw;
     }
-    bd.n_queries = Q;
+    bd.n_queries = bt->Q;
     bd.n_uterms = bt->U;
-    bd.k = k;
+    bd.k = bt->k;
     bd.cap = bt->cap;
-    const uint32_t plan_docs = bt->plan_docs;
-    bd.tile_docs = plan_docs;
-    bd.n_tiles = std::max(1u, (s->doc_count + plan_docs - 1) / plan_docs);
+    bd.tile_docs = bt->plan_docs;
+    bd.n_tiles = std::max(1u, (s->doc_count + bt->plan_docs - 1) / bt->plan_docs);
     bd.thr_key = bt->thr_key;
     bd.topk_count = bt->topk_count;
     bd.lock = bt->lock;
     bd.topk_keys = bt->topk_keys;
     bd.work_counter = bt->work_counter;
     bd.stats = bt->stats;
-    bd.match_count = bd.stats + (size_t)Q * 4;
-    // queries that name a filter need its bitmap on every segment
-    if (!ix->filters.empty() && s->filter_bits.size() < ix->filters.size())
-      return fail(ix, SLG_ERR_INVALID, "segment %u was loaded after its filters were compiled", s->ord);
+    bd.match_count = bd.stats + (size_t)bt->Q * 4;
+  }
 
-    WarpBatchDev wb{};
-    ItemsDev it{};
+  // wb, it and the warp-per-item / items kernels' shared memory and grid
+  int32_t warp_view(ScorePath path) {
+    const bool scan = path == ScorePath::Scan;
+    wb.qterms = bt->qterms;
+    wb.qheads = bt->qheads;
+    wb.rng = bd.ut_rng;
+    wb.sub_ub = bd.ut_tile_ub;
+    wb.scores = s->dev.post_score;
+    wb.filter_bits = bd.filter_bits;
+    wb.n_queries = bt->Q;
+    wb.k = bt->k;
+    wb.sub_docs = bt->plan_docs;
+    wb.q_leaves = bd.q_leaves;
+    wb.q_plan_off = bd.q_plan_off;
+    wb.plan_nodes = bd.plan_nodes;
+    wb.max_leaves = bt->max_leaves;
+    wb.n_sub = bd.n_tiles;
+    wb.n_groups = (bd.n_tiles + kSubPerGroup - 1) / kSubPerGroup;
+    wb.ms_frac = (float)ix->maxscore_pct / 100.0f;
+    wb.thr_key = bd.thr_key;
+    wb.topk_count = bd.topk_count;
+    wb.lock = bd.lock;
+    wb.topk_keys = bd.topk_keys;
+    wb.work_counter = bd.work_counter;
+    wb.stats = bd.stats;
+    wb.match_count = bd.match_count;
+    wb.q_cursor = bd.q_cursor;
+    wb.q_saw = bd.q_saw;
+    wb.pool_keys = scan ? bt->pool_keys : nullptr;
+    wb.pool_count = bt->pool_count;
+    wb.pool_lock = bt->pool_lock;
+    wb.pool_cap = bt->pool_cap;
+    wb.board = scan ? bt->board : nullptr;  // (the posting scan and its column pass read and push; the other kernels keep to themselves)
+    for (uint32_t p = 0; p < kMaxBoardPeers; p++) wb.peer_board[p] = bt->peer_board[p];
+    wb.n_peers = bt->n_board_peers;
+    wb.epoch = bt->board_epoch;
     const int warps = kThreads / 32;
-    size_t wsmem = 0;
-    int wgrid = 1;
-    const bool score = bt->U && s->doc_count;
-    if (bt->use_warp && score) {
-      wb.qterms = bt->qterms;
-      wb.qheads = bt->qheads;
-      wb.rng = bd.ut_rng;
-      wb.sub_ub = bd.ut_tile_ub;
-      wb.scores = s->dev.post_score;
-      wb.filter_bits = bd.filter_bits;
-      wb.n_queries = Q;
-      wb.k = k;
-      wb.sub_docs = plan_docs;
-      wb.q_leaves = bd.q_leaves;
-      wb.q_plan_off = bd.q_plan_off;
-      wb.plan_nodes = bd.plan_nodes;
-      wb.max_leaves = bt->max_leaves;
-      wb.n_sub = bd.n_tiles;
-      wb.n_groups = (bd.n_tiles + kSubPerGroup - 1) / kSubPerGroup;
-      wb.ms_frac = (float)ix->maxscore_pct / 100.0f;
-      wb.thr_key = bd.thr_key;
-      wb.topk_count = bd.topk_count;
-      wb.lock = bd.lock;
-      wb.topk_keys = bd.topk_keys;
-      wb.work_counter = bd.work_counter;
-      wb.stats = bd.stats;
-      wb.match_count = bd.match_count;
-      wb.q_cursor = bd.q_cursor;
-      wb.q_saw = bd.q_saw;
-      wb.pool_keys = run_scan ? bt->pool_keys : nullptr;
-      wb.pool_count = bt->pool_count;
-      wb.pool_lock = bt->pool_lock;
-      wb.pool_cap = bt->pool_cap;
-      wb.board = run_scan ? bt->board : nullptr;  // (the posting scan and its column pass read and push; the other kernels keep to themselves)
-      for (uint32_t p = 0; p < kMaxBoardPeers; p++) wb.peer_board[p] = bt->peer_board[p];
-      wb.n_peers = bt->n_board_peers;
-      wb.epoch = bt->board_epoch;
-      // (plan batches: the matcher form of the kernel unless the staged plain-OR form applies — size for the larger)
-      wsmem = run_items ? (size_t)warps * warp_kernel_smem_per_warp(wb.sub_docs, false, true, 1)
-                        : (size_t)warps * warp_kernel_smem_per_warp(wb.sub_docs, bt->matcher || (bt->has_plan && !bt->staged), prune,
-                                                                    bt->has_plan ? bt->max_leaves : 1u);
-      if (wsmem + 1024 > ix->smem_optin) return fail(ix, SLG_ERR_UNSUPPORTED, "sub_docs %u needs %zu B shared memory", ix->sub_docs, wsmem);
-      uint32_t wper = (uint32_t)std::max<size_t>(1, (ix->smem_optin + 1024) / (wsmem + 1024));
-      wper = std::min(wper, 3u);  // the kernels are compiled for at most 3 CTAs per SM (__launch_bounds__)
-      if (ix->ctas_per_sm) wper = std::min(wper, ix->ctas_per_sm);
-      wgrid = (int)std::min<uint64_t>((uint64_t)ix->n_sm * wper, ((uint64_t)wb.n_groups * wb.n_queries + warps - 1) / warps);
-      it.items = nullptr;
-      it.n_items = bt->n_items;
-      it.done = bt->done;
-      it.items_out = bt->items;
-      it.n_items_out = bt->n_items;
-      it.items_cap = bt->items_cap;
-      it.counters = bt->item_counters;
-    }
+    // (plan batches: the matcher form of the kernel unless the staged plain-OR form applies — size for the larger)
+    const bool walks = scan || path == ScorePath::Stream || path == ScorePath::Items;
+    wsmem = walks ? (size_t)warps * warp_kernel_smem_per_warp(wb.sub_docs, false, true, 1)
+                  : (size_t)warps * warp_kernel_smem_per_warp(wb.sub_docs, bt->matcher || (bt->has_plan && !bt->sel.staged), prune, bt->max_leaves);
+    if (wsmem + 1024 > ix->smem_optin) return fail(ix, SLG_ERR_UNSUPPORTED, "sub_docs %u needs %zu B shared memory", ix->sub_docs, wsmem);
+    const uint32_t wper = ctas_for_smem(ix, wsmem, 3u);  // the kernels are compiled for at most 3 CTAs per SM (__launch_bounds__)
+    wgrid = (int)std::min<uint64_t>((uint64_t)ix->n_sm * wper, ((uint64_t)wb.n_groups * wb.n_queries + warps - 1) / warps);
+    it.n_items = bt->n_items;
+    it.done = bt->done;
+    it.items_out = bt->items;
+    it.n_items_out = bt->n_items;
+    it.items_cap = bt->items_cap;
+    it.counters = bt->item_counters;
+    return SLG_OK;
+  }
 
-    if (do_seeds) {
-      // ---- reset, plans and per-segment query tables ----
-      const uint32_t n_reset = std::max(Q, (uint32_t)(bt->state_bytes / 4));
-      slg_reset_state_kernel<<<(n_reset + 255) / 256, 256, 0, st>>>(bd.thr_key, Q, reinterpret_cast<uint32_t *>(bt->state),
-                                                                    (uint32_t)(bt->state_bytes / 4));
-      count_launch(ix);
-      if (score && run_scan) {
-        // no doc-range plan: the scan walks whole lists and looks terms up by binary search
-        slg_build_qterms_kernel<<<(Q + 127) / 128, 128, 0, st>>>(s->dev, bd, bt->qterms, bt->qheads, bt->canonical, true);
-        count_launch(ix);
-        SLG_CUDA(ix, cudaGetLastError());
-      } else if (score) {
-        const uint64_t n2 = (uint64_t)bt->U * bd.n_tiles;
-        // every unique term: short lists are walked once, long lists take one binary search per boundary.  The items
-        // kernel never walks the postings of a column term, so their rows are not planned for it.
-        slg_plan_walk_kernel<<<dim3(bt->U, 8), 256, 0, st>>>(s->dev, bd.ut_term, nullptr, bt->U, bd.tile_docs, bd.n_tiles, !run_items,
-                                                            bd.ut_rng);
-        count_launch(ix);
-        if (bd.ut_tile_ub && (prune || run_items)) {
-          if (s->dev.mb_max) {
-            slg_items_bounds_kernel<<<(unsigned)((n2 + 255) / 256), 256, 0, st>>>(s->dev, bd.ut_term, bt->U, bd.ut_rng, bd.tile_docs, bd.n_tiles,
-                                                                                 bd.ut_tile_ub);
-          } else {
-            slg_plan_bounds_kernel<<<(unsigned)((n2 + 255) / 256), 256, 0, st>>>(s->dev, bd, nullptr, bt->U);
-          }
-          count_launch(ix);
-        }
-        if (bt->use_warp) {
-          slg_build_qterms_kernel<<<(Q + 127) / 128, 128, 0, st>>>(s->dev, bd, bt->qterms, bt->qheads, bt->canonical, run_items);
-          count_launch(ix);
-        }
-        SLG_CUDA(ix, cudaGetLastError());
+  // the column-pass tables; strict = 1: the sparse pass sums every posting per doc
+  StreamDev stream_view(uint32_t strict) const {
+    StreamDev sdv{};
+    sdv.colq = bt->colq;
+    sdv.n_colq = bt->work_counter + 3;
+    sdv.ucol = bt->ucol;
+    sdv.n_ucol = bt->work_counter + 4;
+    sdv.col_slot = bt->col_slot;
+    sdv.sparse_counter = bt->work_counter + 1;
+    sdv.col_counter = bt->work_counter + 2;
+    sdv.stage_cap = bt->ix->stage_cap;
+    sdv.strict = strict;
+    sdv.counters = bt->item_counters;
+    return sdv;
+  }
+
+  // column pass of the Scan and Stream paths: queries grouped by their first column, then the column terms scored from
+  // their columns
+  int32_t column_pass(StreamDev &sdv) {
+    const bool pools = wb.pool_keys != nullptr;
+    slg_colgroups_kernel<<<1, 1024, 0, st>>>(s->dev, wb, sdv, s->n_cols, prune ? bt->ut_max : nullptr);
+    count_launch(ix);
+    SLG_CUDA(ix, cudaGetLastError());
+    sdv.n_smax = std::min(s->n_cols, kColMaxSlots);
+    const size_t fixed = column_smem(0, sdv.n_smax);
+    const size_t reserve = 2048 + (size_t)kColWarps * 256 * 4;  // (+ the kernel's static shared memory)
+    const size_t budget = ix->smem_optin > fixed + reserve ? ix->smem_optin - fixed - reserve : 0;
+    sdv.col_resident = (uint32_t)std::min<size_t>(s->n_cols, budget / (2 * kColBlock * 4));
+    if (prune) {
+      // few queries keep an essential column term: one warp per (query, slice of the doc range), blocks skipped by col_tmax
+      SLG_CUDA(ix, launch_columns_pruned(pools, s->dev, wb, sdv, (int)((bt->Q * kColSlices + 7) / 8), st));
+    } else {
+      // one CTA per SM: as many columns of a block resident in shared memory (double buffered) as fit
+      const uint32_t n_cblocks = (s->doc_count + kColBlock - 1) / kColBlock;
+      SLG_CUDA(ix, launch_score_columns(false, pools, s->dev, wb, sdv, column_smem(sdv.col_resident, sdv.n_smax),
+                                        (int)std::min<uint32_t>((uint32_t)ix->n_sm, n_cblocks), st));
+    }
+    count_launch(ix);
+    return SLG_OK;
+  }
+
+  // the prologue of the sub-tile paths (all but Scan): doc-range plan, per-tile bounds and the warp tables; then the
+  // scoring time starts (ev[2])
+  int32_t plan(bool walks) {
+    const SegmentDev &sd = s->dev;
+    const uint64_t n2 = (uint64_t)bt->U * bd.n_tiles;
+    // every unique term: short lists are walked once, long lists take one binary search per boundary.  The items
+    // kernel never walks the postings of a column term, so their rows are not planned for it.
+    slg_plan_walk_kernel<<<dim3(bt->U, 8), 256, 0, st>>>(sd, bd.ut_term, nullptr, bt->U, bd.tile_docs, bd.n_tiles, !walks, bd.ut_rng);
+    count_launch(ix);
+    if (bd.ut_tile_ub && (prune || walks)) {
+      if (sd.mb_max) {
+        slg_items_bounds_kernel<<<(unsigned)((n2 + 255) / 256), 256, 0, st>>>(sd, bd.ut_term, bt->U, bd.ut_rng, bd.tile_docs, bd.n_tiles, bd.ut_tile_ub);
+      } else {
+        slg_plan_bounds_kernel<<<(unsigned)((n2 + 255) / 256), 256, 0, st>>>(sd, bd, nullptr, bt->U);
       }
-      if (!(score && run_scan)) SLG_CUDA(ix, cudaEventRecord(ix->ev[2], st));
-      if (score && run_items && prune && !run_scan) {
-        // ---- seeds: every query's best items first ----
-        SLG_CUDA(ix, cudaMemsetAsync(bt->done, 0, (size_t)wb.n_groups * Q, st));
-        const int sgrid = (int)std::min<uint32_t>((uint32_t)ix->n_sm * 3u, (Q + warps - 1) / warps);
+      count_launch(ix);
+    }
+    if (bt->sel.warp_tables) {
+      slg_build_qterms_kernel<<<(bt->Q + 127) / 128, 128, 0, st>>>(sd, bd, bt->qterms, bt->qheads, bt->sel.canonical, walks);
+      count_launch(ix);
+    }
+    SLG_CUDA(ix, cudaGetLastError());
+    SLG_CUDA(ix, cudaEventRecord(ix->ev[2], st));
+    return SLG_OK;
+  }
+
+  // flat posting scan over whole lists, then the column pass
+  int32_t scan(bool do_seeds, bool do_sweep) {
+    ScanDev sc{};
+    sc.ut_term = bd.ut_term;
+    sc.ut_max = bt->ut_max;
+    sc.pairs = bt->scan_pairs;
+    sc.order = bt->scan_order;
+    sc.n_pairs = bt->work_counter + 5;
+    sc.n_items = bt->work_counter + 6;
+    sc.item_start = bt->scan_item_start;
+    sc.items = bt->scan_items;
+    sc.items_cap = bt->scan_items_cap;
+    sc.chunk = bt->scan_chunk;
+    sc.must_mode = bt->sel.and_scan ? 1u : 0u;
+    sc.counter = bt->work_counter + 7;
+    sc.counters = bt->item_counters;
+    if (do_seeds) {
+      // no doc-range plan: the scan walks whole lists and looks terms up by binary search
+      slg_build_qterms_kernel<<<(bt->Q + 127) / 128, 128, 0, st>>>(s->dev, bd, bt->qterms, bt->qheads, bt->sel.canonical, true);
+      count_launch(ix);
+      SLG_CUDA(ix, cudaGetLastError());
+      if (prune && s->dev.term_ub) {
+        slg_term_ub_gather_kernel<<<(bt->U + 255) / 256, 256, 0, st>>>(s->dev, sc, bt->U);
+      } else {  // exhaustive: no index-time bound, the maxima are reduced from the batch's posting scores
+        SLG_CUDA(ix, cudaMemsetAsync(bt->ut_max, 0, (size_t)bt->U * 4, st));
+        slg_term_max_kernel<<<dim3((bt->U + 7) / 8, kMaxSlices), 256, 0, st>>>(s->dev, sc, bt->U);
+      }
+      slg_scan_pairs_kernel<<<(bt->Q + 127) / 128, 128, 0, st>>>(s->dev, wb, sc, ix->dbg);
+      slg_scan_order_kernel<<<1, 1024, 0, st>>>(wb, sc);
+      if (bt->scan_items_cap) slg_scan_items_kernel<<<(bt->scan_items_cap + 255) / 256, 256, 0, st>>>(sc);
+      count_launch(ix, 4);
+      SLG_CUDA(ix, cudaGetLastError());
+      SLG_CUDA(ix, cudaEventRecord(ix->ev[2], st));  // (the scoring time of this path starts here)
+    }
+    // one launch over all items, or (sharded runs) the rarest items first, the threshold exchange, then the rest
+    sc.two_rounds = (ix->dbg & 8u) ? 1u : 0u;
+    sc.part_lo = do_seeds ? 0u : ix->scan_first_part;
+    sc.part_hi = do_sweep ? 256u : ix->scan_first_part;
+    SLG_CUDA(ix, launch_scan(prune, wb.pool_keys != nullptr, s->dev, wb, sc, ix->n_sm * 4, st));
+    count_launch(ix);
+    if (do_sweep && s->n_cols && !(ix->dbg & 4u) && !bt->sel.and_scan) {  // (AND: every result holds the scanned term — there is nothing left for a column pass)
+      StreamDev sdv = stream_view(0);
+      return column_pass(sdv);
+    }
+    return SLG_OK;
+  }
+
+  // exhaustive sub-tile path: sparse pass (staged posting runs), then the column pass
+  int32_t stream(bool do_seeds, bool do_sweep) {
+    if (do_seeds)
+      if (int32_t rc = plan(true)) return rc;
+    if (!do_sweep) return SLG_OK;
+    StreamDev sdv = stream_view(ix->strict_accumulate);
+    const size_t ssmem = (size_t)kSparseWarps * sparse_smem_per_warp(wb.sub_docs, sdv.stage_cap);
+    if (ssmem + 1024 > ix->smem_optin) return fail(ix, SLG_ERR_UNSUPPORTED, "sub_docs %u with stage_cap %u needs %zu B shared memory", wb.sub_docs, sdv.stage_cap, ssmem);
+    const uint32_t sper = ctas_for_smem(ix, ssmem, 2048u / (kSparseWarps * 32u));
+    const int sgrid = (int)std::min<uint64_t>((uint64_t)ix->n_sm * sper, ((uint64_t)wb.n_groups * bt->Q + kSparseWarps - 1) / kSparseWarps);
+    SLG_CUDA(ix, launch_score_sparse(s->dev, wb, sdv, ssmem, sgrid, st));
+    count_launch(ix);
+    return s->n_cols ? column_pass(sdv) : SLG_OK;
+  }
+
+  // posting-driven items kernel; pruned: every query's best items first (seeds), then the items that can still qualify
+  int32_t items(bool do_seeds, bool do_sweep) {
+    if (do_seeds) {
+      if (int32_t rc = plan(true)) return rc;
+      if (prune) {
+        SLG_CUDA(ix, cudaMemsetAsync(bt->done, 0, (size_t)wb.n_groups * bt->Q, st));
+        const int warps = kThreads / 32;
+        const int sgrid = (int)std::min<uint32_t>((uint32_t)ix->n_sm * 3u, (bt->Q + warps - 1) / warps);
         SLG_CUDA(ix, launch_seed_items(s->dev, wb, it, wsmem, sgrid, st));
         count_launch(ix);
       }
     }
-    const bool run_stream = run_items && !prune && bt->colq != nullptr && !run_scan && bt->plan_docs <= 2048;  // (posting numbers of a sub-tile fit 15 bits)
-    if ((do_sweep || do_seeds) && score && run_scan) {
-      ScanDev sc{};
-      sc.ut_term = bd.ut_term;
-      sc.ut_max = bt->ut_max;
-      sc.pairs = bt->scan_pairs;
-      sc.order = bt->scan_order;
-      sc.n_pairs = bt->work_counter + 5;
-      sc.n_items = bt->work_counter + 6;
-      sc.item_start = bt->scan_item_start;
-      sc.items = bt->scan_items;
-      sc.items_cap = bt->scan_items_cap;
-      sc.chunk = bt->scan_chunk;
-      sc.must_mode = bt->and_scan ? 1u : 0u;
-      sc.counter = bt->work_counter + 7;
-      sc.counters = bt->item_counters;
-      StreamDev sdv{};
-      sdv.colq = bt->colq;
-      sdv.n_colq = bt->work_counter + 3;
-      sdv.ucol = bt->ucol;
-      sdv.n_ucol = bt->work_counter + 4;
-      sdv.col_slot = bt->col_slot;
-      sdv.sparse_counter = bt->work_counter + 1;
-      sdv.col_counter = bt->work_counter + 2;
-      sdv.stage_cap = ix->stage_cap;
-      sdv.strict = 0;
-      sdv.counters = bt->item_counters;
-      if (do_seeds) {
-        if (prune && s->dev.term_ub) {
-          slg_term_ub_gather_kernel<<<(bt->U + 255) / 256, 256, 0, st>>>(s->dev, sc, bt->U);
-        } else {  // exhaustive: no index-time bound, the maxima are reduced from the batch's posting scores
-          SLG_CUDA(ix, cudaMemsetAsync(bt->ut_max, 0, (size_t)bt->U * 4, st));
-          slg_term_max_kernel<<<dim3((bt->U + 7) / 8, kMaxSlices), 256, 0, st>>>(s->dev, sc, bt->U);
-        }
-        slg_scan_pairs_kernel<<<(Q + 127) / 128, 128, 0, st>>>(s->dev, wb, sc, ix->dbg);
-        slg_scan_order_kernel<<<1, 1024, 0, st>>>(wb, sc);
-        if (bt->scan_items_cap) slg_scan_items_kernel<<<(bt->scan_items_cap + 255) / 256, 256, 0, st>>>(sc);
-        for (int i = 0; i < 4; i++) count_launch(ix);
-        SLG_CUDA(ix, cudaGetLastError());
-        SLG_CUDA(ix, cudaEventRecord(ix->ev[2], st));  // (the scoring time of this path starts here)
-      }
-      // one launch over all items, or (sharded runs) the rarest items first, the threshold exchange, then the rest
-      sc.two_rounds = (ix->dbg & 8u) ? 1u : 0u;
-      sc.part_lo = do_seeds ? 0u : ix->scan_first_part;
-      sc.part_hi = do_sweep ? 256u : ix->scan_first_part;
-      SLG_CUDA(ix, launch_scan(prune, wb.pool_keys != nullptr, s->dev, wb, sc, ix->n_sm * 4, st));
+    if (!do_sweep) return SLG_OK;
+    if (prune) {
+      const uint32_t total = wb.n_groups * bt->Q;
+      slg_filter_items_kernel<<<(total + 255) / 256, 256, 0, st>>>(wb, it);
       count_launch(ix);
-      if (do_sweep && s->n_cols && !(ix->dbg & 4u) && !bt->and_scan) {  // (AND: every result holds the scanned term — there is nothing left for a column pass)
-        slg_colgroups_kernel<<<1, 1024, 0, st>>>(s->dev, wb, sdv, s->n_cols, prune ? bt->ut_max : nullptr);
-        count_launch(ix);
-        SLG_CUDA(ix, cudaGetLastError());
-        sdv.n_smax = std::min(s->n_cols, kColMaxSlots);
-        const size_t fixed = column_smem(0, sdv.n_smax);
-        const size_t reserve = 2048 + (size_t)kColWarps * 256 * 4;  // (+ the kernel's static shared memory)
-        const size_t budget = ix->smem_optin > fixed + reserve ? ix->smem_optin - fixed - reserve : 0;
-        sdv.col_resident = (uint32_t)std::min<size_t>(s->n_cols, budget / (2 * kColBlock * 4));
-        const size_t csmem = column_smem(sdv.col_resident, sdv.n_smax);
-        const uint32_t n_cblocks = (s->doc_count + kColBlock - 1) / kColBlock;
-        if (prune) {
-          // few queries keep an essential column term: one warp per (query, slice of the doc range), blocks skipped by col_tmax
-          (void)csmem;
-          (void)n_cblocks;
-          SLG_CUDA(ix, launch_columns_pruned(wb.pool_keys != nullptr, s->dev, wb, sdv, (int)((Q * kColSlices + 7) / 8), st));
-        } else {
-          SLG_CUDA(ix, launch_score_columns(false, wb.pool_keys != nullptr, s->dev, wb, sdv, csmem, (int)std::min<uint32_t>((uint32_t)ix->n_sm, n_cblocks), st));
-        }
-        count_launch(ix);
-      }
-      if (do_sweep) ix->ctr.score_launches++;
+      SLG_CUDA(ix, cudaGetLastError());
+      it.items = bt->items;
     }
-    if (do_sweep) {
-      // ---- scoring ----
-      if (score && run_scan) {
-        // (launched above)
-      } else if (score && run_stream) {
-        // exhaustive: sparse pass (staged posting runs), then column pass (queries grouped by their first column)
-        StreamDev sdv{};
-        sdv.colq = bt->colq;
-        sdv.n_colq = bt->work_counter + 3;
-        sdv.ucol = bt->ucol;
-        sdv.n_ucol = bt->work_counter + 4;
-        sdv.col_slot = bt->col_slot;
-        sdv.sparse_counter = bt->work_counter + 1;
-        sdv.col_counter = bt->work_counter + 2;
-        sdv.stage_cap = ix->stage_cap;
-        sdv.strict = ix->strict_accumulate;
-        sdv.counters = bt->item_counters;
-        const size_t ssmem = (size_t)kSparseWarps * sparse_smem_per_warp(wb.sub_docs, sdv.stage_cap);
-        if (ssmem + 1024 > ix->smem_optin) return fail(ix, SLG_ERR_UNSUPPORTED, "sub_docs %u with stage_cap %u needs %zu B shared memory", wb.sub_docs, sdv.stage_cap, ssmem);
-        uint32_t sper = (uint32_t)std::max<size_t>(1, (ix->smem_optin + 1024) / (ssmem + 1024));
-        sper = std::min(sper, 2048u / (kSparseWarps * 32u));
-        if (ix->ctas_per_sm) sper = std::min(sper, ix->ctas_per_sm);
-        const int sgrid = (int)std::min<uint64_t>((uint64_t)ix->n_sm * sper, ((uint64_t)wb.n_groups * Q + kSparseWarps - 1) / kSparseWarps);
-        SLG_CUDA(ix, launch_score_sparse(s->dev, wb, sdv, ssmem, sgrid, st));
-        count_launch(ix);
-        if (s->n_cols) {
-          slg_colgroups_kernel<<<1, 1024, 0, st>>>(s->dev, wb, sdv, s->n_cols, nullptr);
-          count_launch(ix);
-          SLG_CUDA(ix, cudaGetLastError());
-          // one CTA per SM: as many columns of a block resident in shared memory (double buffered) as fit
-          sdv.n_smax = std::min(s->n_cols, kColMaxSlots);
-          const size_t fixed = column_smem(0, sdv.n_smax);
-          const size_t reserve = 2048 + (size_t)kColWarps * 256 * 4;  // (+ the kernel's static shared memory)
-        const size_t budget = ix->smem_optin > fixed + reserve ? ix->smem_optin - fixed - reserve : 0;
-          sdv.col_resident = (uint32_t)std::min<size_t>(s->n_cols, budget / (2 * kColBlock * 4));
-          const size_t csmem = column_smem(sdv.col_resident, sdv.n_smax);
-          const uint32_t n_cblocks = (s->doc_count + kColBlock - 1) / kColBlock;
-          SLG_CUDA(ix, launch_score_columns(false, wb.pool_keys != nullptr, s->dev, wb, sdv, csmem, (int)std::min<uint32_t>((uint32_t)ix->n_sm, n_cblocks), st));
-          count_launch(ix);
-        }
-        ix->ctr.score_launches++;
-      } else if (score && run_items) {
-        if (prune) {
-          const uint32_t total = wb.n_groups * Q;
-          slg_filter_items_kernel<<<(total + 255) / 256, 256, 0, st>>>(wb, it);
-          count_launch(ix);
-          SLG_CUDA(ix, cudaGetLastError());
-          it.items = bt->items;
-        }
-        SLG_CUDA(ix, launch_score_items(prune, s->dev, wb, it, wsmem, wgrid, st));
-        count_launch(ix);
-        ix->ctr.score_launches++;
-      } else if (score && warp_path) {
-        SLG_CUDA(ix, launch_score_warp(bt->matcher, prune, bt->want_stats, bt->staged, bt->has_plan, s->dev, wb, wsmem, wgrid, st));
-        count_launch(ix);
-        ix->ctr.score_launches++;
-      } else if (score) {
-        int grid = (int)std::min<uint64_t>((uint64_t)ix->n_sm * per_sm, (uint64_t)bd.n_tiles * Q);
-        SLG_CUDA(ix, launch_score_tiles(bt->matcher, prune, bt->want_stats, bt->has_plan, s->dev, bd, smem, grid, st));
-        count_launch(ix);
-        ix->ctr.score_launches++;
+    SLG_CUDA(ix, launch_score_items(prune, s->dev, wb, it, wsmem, wgrid, st));
+    count_launch(ix);
+    return SLG_OK;
+  }
+};
+
+int32_t finish_timing(slg_batch *bt) {
+  slg_index *ix = bt->ix;
+  SLG_CUDA(ix, cudaStreamSynchronize(ix->stream));
+  float ms = 0;
+  SLG_CUDA(ix, cudaEventElapsedTime(&ms, ix->ev[0], ix->ev[1]));
+  ix->ctr.last_batch_ms = ms;
+  if (ix->segs.size() == 1 && bt->U) {
+    SLG_CUDA(ix, cudaEventElapsedTime(&ms, ix->ev[2], ix->ev[3]));
+    ix->ctr.score_ms_total += ms;
+    ix->ctr.last_score_ms = ms;
+  }
+  return SLG_OK;
+}
+
+// everything of one run up to (seeds_only) or including the sweep; see the schedule in slg_batch_run
+int32_t run_batch(slg_batch *bt, bool do_seeds, bool do_sweep, int32_t sync) {
+  slg_index *ix = bt->ix;
+  SLG_CUDA(ix, cudaSetDevice(ix->device));
+  cudaStream_t st = ix->stream;
+  const bool prune = bt->exec != SLG_EXEC_BM25;
+  const uint32_t Q = bt->Q, k = bt->k;
+  RunFacts rf;
+  rf.want_stats = bt->want_stats;
+  rf.prune = prune;
+  rf.scan_kernels = ix->scan_kernels;
+  rf.strict_accumulate = ix->strict_accumulate;
+  rf.small_plan_docs = bt->plan_docs <= 2048;
+  rf.two_step = !(do_seeds && do_sweep);
+  rf.one_segment = ix->segs.size() == 1;
+  ScorePath path = ScorePath::Tiles;
+  if (const char *why = choose_path(bt->sel, rf, path)) return fail(ix, SLG_ERR_UNSUPPORTED, "%s", why);
+  size_t smem = 0;  // (max_leaves is 1 without a plan)
+  if (path == ScorePath::Tiles)
+    if (int32_t rc = select_smem(ix, bt->has_plan ? bt->plan_docs : ix->tile_docs, bt->cap, bt->matcher, &smem, bt->max_leaves)) return rc;
+  if (do_seeds) {
+    SLG_CUDA(ix, cudaEventRecord(ix->ev[0], st));
+    SLG_CUDA(ix, cudaMemsetAsync(bt->stats, 0, (size_t)Q * 40 + 64, st));
+    if (bt->has_cursor) {
+      if (bt->n_cursor_segs != ix->segs.size()) return fail(ix, SLG_ERR_INVALID, "a segment was loaded after the batch with cursors was prepared");
+      SLG_CUDA(ix, cudaMemsetAsync(bt->cursor_saw, 0, (size_t)Q * 4, st));
+    }
+  }
+  uint32_t si = 0;
+  for (auto &sp : ix->segs) {
+    SegmentRun v{bt, ix, st, prune, sp.get()};
+    // queries that name a filter need its bitmap on every segment
+    if (!ix->filters.empty() && v.s->filter_bits.size() < ix->filters.size())
+      return fail(ix, SLG_ERR_INVALID, "segment %u was loaded after its filters were compiled", v.s->ord);
+    v.batch_view(si);
+    const bool score = bt->U && v.s->doc_count;
+    if (bt->sel.warp_tables && score)
+      if (int32_t rc = v.warp_view(path)) return rc;
+
+    if (do_seeds) {
+      const uint32_t n_reset = std::max(Q, (uint32_t)(bt->state_bytes / 4));
+      slg_reset_state_kernel<<<(n_reset + 255) / 256, 256, 0, st>>>(v.bd.thr_key, Q, reinterpret_cast<uint32_t *>(bt->state),
+                                                                    (uint32_t)(bt->state_bytes / 4));
+      count_launch(ix);
+    }
+    int32_t rc = SLG_OK;
+    if (!score) {
+      if (do_seeds) SLG_CUDA(ix, cudaEventRecord(ix->ev[2], st));
+    } else {
+      switch (path) {
+        case ScorePath::Scan: rc = v.scan(do_seeds, do_sweep); break;
+        case ScorePath::Stream: rc = v.stream(do_seeds, do_sweep); break;
+        case ScorePath::Items: rc = v.items(do_seeds, do_sweep); break;
+        case ScorePath::Warp:
+          if (do_seeds) rc = v.plan(false);
+          if (do_sweep && !rc) {
+            SLG_CUDA(ix, launch_score_warp(bt->matcher, prune, bt->want_stats, bt->sel.staged, bt->has_plan, v.s->dev, v.wb, v.wsmem, v.wgrid, st));
+            count_launch(ix);
+          }
+          break;
+        case ScorePath::Tiles:
+          if (do_seeds) rc = v.plan(false);
+          if (do_sweep && !rc) {
+            const int grid = (int)std::min<uint64_t>((uint64_t)ix->n_sm * ctas_for_smem(ix, smem, 8u), (uint64_t)v.bd.n_tiles * Q);
+            SLG_CUDA(ix, launch_score_tiles(bt->matcher, prune, bt->want_stats, bt->has_plan, v.s->dev, v.bd, smem, grid, st));
+            count_launch(ix);
+          }
+          break;
       }
+    }
+    if (rc) return rc;
+    if (do_sweep) {
+      if (score) ix->ctr.score_launches++;  // one per segment scored, whichever path
       SLG_CUDA(ix, cudaEventRecord(ix->ev[3], st));
       HitDev *hits = reinterpret_cast<HitDev *>(bt->results + (size_t)si * bt->result_stride);
       uint32_t *cnts = reinterpret_cast<uint32_t *>(bt->results + (size_t)si * bt->result_stride + (size_t)Q * k * sizeof(HitDev));
       size_t fsmem = (size_t)(1u << (32 - __builtin_clz(std::max(k, 2u) - 1))) * 8;
-      if (run_scan && bt->pool_keys && score) {
+      if (path == ScorePath::Scan && bt->pool_keys && score) {
         const size_t psmem = (size_t)bt->pool_cap * 2 * 8;
         SLG_CUDA(ix, cudaFuncSetAttribute(slg_finalize_pools_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)psmem));
-        slg_finalize_pools_kernel<<<Q, kThreads, psmem, st>>>(bt->pool_keys, bt->pool_count, bt->pool_cap, k, s->ord, hits, cnts);
+        slg_finalize_pools_kernel<<<Q, kThreads, psmem, st>>>(bt->pool_keys, bt->pool_count, bt->pool_cap, k, v.s->ord, hits, cnts);
       } else {
-        slg_finalize_kernel<<<Q, kThreads, fsmem, st>>>(bd, s->ord, hits, cnts);
+        slg_finalize_kernel<<<Q, kThreads, fsmem, st>>>(v.bd, v.s->ord, hits, cnts);
       }
       count_launch(ix);
       SLG_CUDA(ix, cudaGetLastError());
@@ -793,46 +790,18 @@ int32_t run_batch(slg_batch *bt, bool do_seeds, bool do_sweep) {
     SLG_CUDA(ix, cudaEventRecord(ix->ev[1], st));
     ix->ctr.last_posting_count = bt->posting_count;
   }
-  return SLG_OK;
+  bt->seeds_done = !do_sweep;
+  return do_sweep && sync ? finish_timing(bt) : SLG_OK;
 }
 
-int32_t finish_timing(slg_batch *bt) {
-  slg_index *ix = bt->ix;
-  SLG_CUDA(ix, cudaStreamSynchronize(ix->stream));
-  float ms = 0;
-  SLG_CUDA(ix, cudaEventElapsedTime(&ms, ix->ev[0], ix->ev[1]));
-  ix->ctr.last_batch_ms = ms;
-  if (ix->segs.size() == 1 && bt->U) {
-    SLG_CUDA(ix, cudaEventElapsedTime(&ms, ix->ev[2], ix->ev[3]));
-    ix->ctr.score_ms_total += ms;
-    ix->ctr.last_score_ms = ms;
-  }
-  return SLG_OK;
-}
 
 }  // namespace
 
 extern "C" {
 
-int32_t slg_batch_run(slg_batch_t *bt, int32_t sync) {
-  if (!bt) return SLG_ERR_INVALID;
-  slg_index *ix = bt->ix;
-  SLG_CUDA(ix, cudaSetDevice(ix->device));
-  int32_t rc = run_batch(bt, true, true);
-  if (rc) return rc;
-  bt->seeds_done = false;
-  return sync ? finish_timing(bt) : SLG_OK;
-}
+int32_t slg_batch_run(slg_batch_t *bt, int32_t sync) { return bt ? run_batch(bt, true, true, sync) : SLG_ERR_INVALID; }
 
-int32_t slg_batch_run_seeds(slg_batch_t *bt) {
-  if (!bt) return SLG_ERR_INVALID;
-  slg_index *ix = bt->ix;
-  SLG_CUDA(ix, cudaSetDevice(ix->device));
-  int32_t rc = run_batch(bt, true, false);
-  if (rc) return rc;
-  bt->seeds_done = true;
-  return SLG_OK;
-}
+int32_t slg_batch_run_seeds(slg_batch_t *bt) { return bt ? run_batch(bt, true, false, 0) : SLG_ERR_INVALID; }
 
 int32_t slg_batch_threshold_keys(slg_batch_t *bt, void **dev_keys) {
   if (!bt || !dev_keys) return SLG_ERR_INVALID;
@@ -853,13 +822,8 @@ int32_t slg_batch_import_thresholds(slg_batch_t *bt, const void *dev_keys) {
 
 int32_t slg_batch_run_sweep(slg_batch_t *bt, int32_t sync) {
   if (!bt) return SLG_ERR_INVALID;
-  slg_index *ix = bt->ix;
-  if (!bt->seeds_done) return fail(ix, SLG_ERR_INVALID, "slg_batch_run_sweep follows slg_batch_run_seeds");
-  SLG_CUDA(ix, cudaSetDevice(ix->device));
-  int32_t rc = run_batch(bt, false, true);
-  if (rc) return rc;
-  bt->seeds_done = false;
-  return sync ? finish_timing(bt) : SLG_OK;
+  if (!bt->seeds_done) return fail(bt->ix, SLG_ERR_INVALID, "slg_batch_run_sweep follows slg_batch_run_seeds");
+  return run_batch(bt, false, true, sync);
 }
 
 int32_t slg_batch_set_threshold_board(slg_batch_t *bt, void *local_board, void *const *peer_boards, uint32_t n_peers, uint32_t epoch) {
