@@ -15,7 +15,7 @@ cudaError_t launch_score_items(bool prune, const SegmentDev &sd, const WarpBatch
 cudaError_t launch_score_sparse(const SegmentDev &sd, const WarpBatchDev &wb, const StreamDev &st_dev, size_t smem, int grid, cudaStream_t st);
 cudaError_t launch_score_columns(bool prune, bool pools, const SegmentDev &sd, const WarpBatchDev &wb, const StreamDev &st_dev, size_t smem, int grid, cudaStream_t st);
 cudaError_t launch_scan(bool prune, bool pools, const SegmentDev &sd, const WarpBatchDev &wb, const ScanDev &sc, int grid, cudaStream_t st);
-cudaError_t launch_columns_pruned(bool pools, const SegmentDev &sd, const WarpBatchDev &wb, const StreamDev &st_dev, int grid, cudaStream_t st);
+cudaError_t launch_columns_ordered(bool pools, const SegmentDev &sd, const WarpBatchDev &wb, const StreamDev &st_dev, int grid, cudaStream_t st);
 cudaError_t launch_seed_items(const SegmentDev &sd, const WarpBatchDev &wb, const ItemsDev &it, size_t smem, int grid, cudaStream_t st);
 
 }  // namespace slg

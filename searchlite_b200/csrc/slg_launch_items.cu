@@ -37,9 +37,9 @@ cudaError_t launch_score_columns(bool prune, bool pools, const SegmentDev &sd, c
   return prune ? go_n(slg_score_columns_kernel<true, false>, kColWarps * 32, smem, grid, st, sd, wb, st_dev)
                : go_n(slg_score_columns_kernel<false, false>, kColWarps * 32, smem, grid, st, sd, wb, st_dev);
 }
-cudaError_t launch_columns_pruned(bool pools, const SegmentDev &sd, const WarpBatchDev &wb, const StreamDev &st_dev, int grid, cudaStream_t st) {
-  if (pools) slg_columns_pruned_kernel<1><<<grid, 256, 0, st>>>(sd, wb, st_dev);
-  else slg_columns_pruned_kernel<0><<<grid, 256, 0, st>>>(sd, wb, st_dev);
+cudaError_t launch_columns_ordered(bool pools, const SegmentDev &sd, const WarpBatchDev &wb, const StreamDev &st_dev, int grid, cudaStream_t st) {
+  if (pools) slg_columns_ordered_kernel<1><<<grid, 256, 0, st>>>(sd, wb, st_dev);
+  else slg_columns_ordered_kernel<0><<<grid, 256, 0, st>>>(sd, wb, st_dev);
   return cudaGetLastError();
 }
 template <bool PRUNE, bool POOLS>

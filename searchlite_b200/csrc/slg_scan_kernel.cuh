@@ -103,97 +103,187 @@ static __global__ void slg_term_ub_gather_kernel(SegmentDev seg, ScanDev sc, uin
   sc.ut_max[u] = term < seg.n_terms ? seg.term_ub[term] : 0.0f;
 }
 
-// pruned executions: the column terms of the few queries that still have an essential one.  Warp per (query, slice of
-// the doc range): 32 blocks of 512 docs at a time, lane = block: the sum of the columns' exact block maxima (seg.col_tmax,
-// slot order) + extra below the k-th score means no doc of the block can enter the top k and the block is not read; the
-// others are summed per doc (16 docs per lane, slot order) and the docs that can still qualify are verified exactly.
-constexpr uint32_t kColSlices = 64;
+// pruned executions: the column terms of the queries that still have an essential one after the scan.  kColParts CTAs per
+// query: CTA `part` takes every kColParts-th chunk of 32 blocks of 512 docs of the segment, from chunk `part`, so that no
+// query's blocks wait on one CTA.  A block's bound
+// is the sum of its columns' exact block maxima (seg.col_tmax, slot order); bound + extra below the k-th score means no
+// doc of the block can enter the top k and the block is not read.  A CTA visits its blocks in DESCENDING order of their bound, so the blocks most
+// likely to hold the top k are scored first and the k-th score is close to final before the bulk comes up: a 256-bin
+// histogram of the bounds (linear from 0 to the same sum over the columns' whole maxima, ut_max), then rounds, each
+// taking the highest bins left (at least kColRound << round blocks) and sweeping the CTA's chunks for their blocks.  Bins
+// are monotone in the bound, so a CTA ends once the largest bound left is below the k-th score.  An open block is
+// summed per doc (16 docs per lane, slot order), the docs that can still qualify are verified exactly and offered, and
+// the warps share their k-th key through shared memory after every block, and through the query's threshold, which every
+// CTA of the query reads before every chunk, after every round.
+constexpr uint32_t kColParts = 8;   // CTAs per query
+constexpr uint32_t kColRound = 64;  // blocks of a CTA's first round; every further round at least doubles
 // POOLS: k > kWarpMaxK (candidate pools + radix select); compiled out otherwise so that the common small-k kernels stay lean
 template <int POOLS>
-__global__ void __launch_bounds__(256) slg_columns_pruned_kernel(SegmentDev seg, WarpBatchDev wb, StreamDev sd) {
+__global__ void __launch_bounds__(256) slg_columns_ordered_kernel(SegmentDev seg, WarpBatchDev wb, StreamDev sd) {
   __shared__ __align__(16) unsigned long long s_cand[8][kWarpCand];
   __shared__ uint32_t s_hist[8][POOLS ? 256 : 1];
+  __shared__ uint32_t s_bin_n[256], s_bin_max[256];  // blocks per bin and the largest bound (bits) of each
+  __shared__ int s_lo, s_hi;                         // the round's bins
+  __shared__ uint32_t s_next, s_open;
+  __shared__ unsigned long long s_thr;               // the best k-th key a warp of the CTA has found
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const uint32_t n_colq = *sd.n_colq;
-  const uint32_t wid = blockIdx.x * 8 + warp;
-  const uint32_t qidx = wid / kColSlices, slice = wid % kColSlices;
-  if (qidx >= n_colq) return;
+  const uint32_t qidx = blockIdx.x / kColParts, part = blockIdx.x % kColParts;
+  if (qidx >= *sd.n_colq) return;
+  const uint32_t n_blocks = (seg.doc_count + 511u) >> 9, n_chunks = (n_blocks + 31u) >> 5;
   const ColQ cq = sd.colq[qidx];
   const QTerm *qts = wb.qterms + (uint64_t)cq.qslot * kWarpMaxTerms;
   const uint32_t nt = (uint32_t)cq.nsp + cq.ncol;
-  const uint32_t n_blocks = (seg.doc_count + 511u) >> 9;
-  const uint32_t per = (n_blocks + kColSlices - 1) / kColSlices;
-  const uint32_t b0 = slice * per, b1 = min(n_blocks, b0 + per);
+  const uint32_t my_chunks = n_chunks > part ? (n_chunks - part + kColParts - 1) / kColParts : 0u;
   WarpCand wc;
   wc.begin(s_cand[warp], load_threshold(wb, cq.qi), wb.k, lane, 1u, POOLS ? s_hist[warp] : nullptr);
-  auto cut_of = [&]() {
-    if (wc.thr == kThrInit) return 0u;
-    const float cf = __uint_as_float((uint32_t)(wc.thr >> 32)) * 0.99998f - cq.extra * 1.00002f;
+  auto cut_from = [&](unsigned long long thr) {
+    if (thr == kThrInit) return 0u;
+    const float cf = __uint_as_float((uint32_t)(thr >> 32)) * 0.99998f - cq.extra * 1.00002f;
     return cf > 0.0f ? __float_as_uint(cf) : 0u;
   };
-  for (uint32_t bb = b0; bb < b1; bb += 32) {
-    const uint32_t blk = bb + lane;
+  auto bound_of = [&](uint32_t blk) {
     float bound = 0.0f;
-    if (blk < b1)
-      for (uint32_t i = 0; i < cq.ncol; i++) {
-        const QTerm &q = qts[cq.nsp + i];
-        bound = __fadd_rn(bound, __fmul_rn(__ldg(seg.col_tmax + (uint64_t)q.term * seg.tmax_stride + blk), q.weight));
-      }
-    uint32_t open = __ballot_sync(0xFFFFFFFFu, blk < b1 && bound != 0.0f && __float_as_uint(bound) >= cut_of());
-    while (open) {
-      const uint32_t d0 = (bb + (__ffs(open) - 1)) << 9;
-      open &= open - 1;
-      float4 v[4];
-#pragma unroll
-      for (int x = 0; x < 4; x++) v[x] = make_float4(0, 0, 0, 0);
-      for (uint32_t i = 0; i < cq.ncol; i++) {
-        const QTerm &q = qts[cq.nsp + i];
-        const float4 *p = reinterpret_cast<const float4 *>(seg.cols + q.sc_base + d0) + lane;
-        const float w = q.weight;
-#pragma unroll
-        for (int x = 0; x < 4; x++) {
-          const float4 c = __ldg(p + x * 32);
-          v[x].x = __fadd_rn(v[x].x, __fmul_rn(c.x, w));
-          v[x].y = __fadd_rn(v[x].y, __fmul_rn(c.y, w));
-          v[x].z = __fadd_rn(v[x].z, __fmul_rn(c.z, w));
-          v[x].w = __fadd_rn(v[x].w, __fmul_rn(c.w, w));
-        }
-      }
-      uint32_t cut = cut_of();
-      uint32_t todo = 0u;
-#pragma unroll
-      for (int x = 0; x < 4; x++) {
-        const uint32_t bx[4] = {__float_as_uint(v[x].x), __float_as_uint(v[x].y), __float_as_uint(v[x].z), __float_as_uint(v[x].w)};
-#pragma unroll
-        for (int e = 0; e < 4; e++)
-          if (bx[e] >= cut && bx[e] != 0u && d0 + x * 128 + lane * 4 + e < seg.doc_count) todo |= 1u << (x * 4 + e);
-      }
-      while (__any_sync(0xFFFFFFFFu, todo != 0u)) {
-        const uint32_t el = todo ? __ffs(todo) - 1 : 0u;
-        const bool had = todo != 0u;
-        todo &= todo - 1u;
-        uint32_t bits = 0u;
-#pragma unroll
-        for (int x = 0; x < 4; x++) {
-          if (el == (uint32_t)x * 4 + 0) bits = __float_as_uint(v[x].x);
-          if (el == (uint32_t)x * 4 + 1) bits = __float_as_uint(v[x].y);
-          if (el == (uint32_t)x * 4 + 2) bits = __float_as_uint(v[x].z);
-          if (el == (uint32_t)x * 4 + 3) bits = __float_as_uint(v[x].w);
-        }
-        const uint32_t doc = d0 + (el >> 2) * 128 + lane * 4 + (el & 3u);
-        cut = cut_of();
-        const bool pass = had && bits >= cut;
-        if (!__any_sync(0xFFFFFFFFu, pass)) continue;
-        float s = __uint_as_float(bits);
-        if (cq.nsp) {
-          uint32_t holders = 0u;
-          s = verify_doc(seg, wb, qts, nt, pass, doc, holders);  // (a sparse list the scan dropped may hold the doc)
-        }
-        wc.offer(seg, wb, cq.qi, cq.filter, pass, doc, s);
-      }
+    for (uint32_t i = 0; i < cq.ncol; i++) {
+      const QTerm &q = qts[cq.nsp + i];
+      bound = __fadd_rn(bound, __fmul_rn(__ldg(seg.col_tmax + (uint64_t)q.term * seg.tmax_stride + blk), q.weight));
+    }
+    return bound;
+  };
+  float top = 0.0f;
+  for (uint32_t i = 0; i < cq.ncol; i++) {
+    const QTerm &q = qts[cq.nsp + i];
+    top = __fadd_rn(top, __fmul_rn(__ldg(sd.ut_max + q.uterm), q.weight));
+  }
+  const float scale = top > 0.0f ? 256.0f / top : 0.0f;
+  auto bin_of = [&](float bound) { return min(255u, __float2uint_rz(__fmul_rn(bound, scale))); };
+  auto block_of = [&](uint32_t i) { return ((part + (i >> 5) * kColParts) << 5) + (i & 31u); };  // i-th block of the CTA
+
+  // ---- the histogram of the bounds that reach the k-th score the pass starts from
+  s_bin_n[threadIdx.x] = 0u;
+  s_bin_max[threadIdx.x] = 0u;
+  if (threadIdx.x == 0) {
+    s_open = 0u;
+    s_thr = wc.thr;
+  }
+  __syncthreads();
+  {
+    const uint32_t cut0 = cut_from(wc.thr);
+    for (uint32_t i = threadIdx.x; i < my_chunks * 32u; i += blockDim.x) {
+      const uint32_t blk = block_of(i);
+      if (blk >= n_blocks) continue;
+      const float bound = bound_of(blk);
+      if (bound == 0.0f || __float_as_uint(bound) < cut0) continue;
+      const uint32_t bin = bin_of(bound);
+      atomicAdd(&s_bin_n[bin], 1u);
+      atomicMax(&s_bin_max[bin], __float_as_uint(bound));
+      atomicAdd(&s_open, 1u);
     }
   }
-  wc.merge(wb, cq.qi);
+  // ---- rounds, highest bins first
+  uint32_t n_scored = 0;
+  int next_bin = 255;
+  for (uint32_t round = 0;; round++) {
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      s_thr = max(s_thr, load_threshold(wb, cq.qi));
+      const uint32_t cut = cut_from(s_thr);
+      int hi = next_bin;
+      while (hi >= 0 && s_bin_n[hi] == 0u) hi--;
+      int lo = hi;
+      if (hi >= 0 && s_bin_max[hi] >= cut) {
+        const uint32_t want = kColRound << min(round, 16u);
+        uint32_t take = s_bin_n[hi];
+        while (lo > 0 && take < want) {
+          if (s_bin_n[lo - 1] && s_bin_max[lo - 1] < cut) break;  // (it and every bin below it are done)
+          take += s_bin_n[--lo];
+        }
+      } else {
+        hi = -1;
+      }
+      s_lo = lo;
+      s_hi = hi;
+      s_next = 0u;
+    }
+    __syncthreads();
+    const int lo = s_lo, hi = s_hi;
+    if (hi < 0) break;
+    next_bin = lo - 1;
+    for (;;) {
+      uint32_t c = 0u;
+      if (lane == 0) c = atomicAdd(&s_next, 1u);
+      c = __shfl_sync(0xFFFFFFFFu, c, 0);
+      if (c >= my_chunks) break;
+      const uint32_t bb = block_of(c << 5), blk = bb + lane;
+      const float bound = blk < n_blocks ? bound_of(blk) : 0.0f;
+      const int bin = (int)bin_of(bound);
+      wc.thr = max(wc.thr, max(*(volatile unsigned long long *)&s_thr, load_threshold(wb, cq.qi)));
+      uint32_t open = __ballot_sync(0xFFFFFFFFu, bound != 0.0f && bin >= lo && bin <= hi && __float_as_uint(bound) >= cut_from(wc.thr));
+      while (open) {
+        const int j = __ffs(open) - 1;
+        open &= open - 1;
+        // (the block before, or another warp, may have raised the k-th score)
+        wc.thr = max(wc.thr, *(volatile unsigned long long *)&s_thr);
+        if (__shfl_sync(0xFFFFFFFFu, __float_as_uint(bound), j) < cut_from(wc.thr)) continue;
+        n_scored++;
+        const uint32_t d0 = (bb + j) << 9;
+        float4 v[4];
+#pragma unroll
+        for (int x = 0; x < 4; x++) v[x] = make_float4(0, 0, 0, 0);
+        for (uint32_t i = 0; i < cq.ncol; i++) {
+          const QTerm &q = qts[cq.nsp + i];
+          const float4 *p = reinterpret_cast<const float4 *>(seg.cols + q.sc_base + d0) + lane;
+          const float w = q.weight;
+#pragma unroll
+          for (int x = 0; x < 4; x++) {
+            const float4 cv = __ldg(p + x * 32);
+            v[x].x = __fadd_rn(v[x].x, __fmul_rn(cv.x, w));
+            v[x].y = __fadd_rn(v[x].y, __fmul_rn(cv.y, w));
+            v[x].z = __fadd_rn(v[x].z, __fmul_rn(cv.z, w));
+            v[x].w = __fadd_rn(v[x].w, __fmul_rn(cv.w, w));
+          }
+        }
+        uint32_t cut = cut_from(wc.thr);
+        uint32_t todo = 0u;
+#pragma unroll
+        for (int x = 0; x < 4; x++) {
+          const uint32_t bx[4] = {__float_as_uint(v[x].x), __float_as_uint(v[x].y), __float_as_uint(v[x].z), __float_as_uint(v[x].w)};
+#pragma unroll
+          for (int e = 0; e < 4; e++)
+            if (bx[e] >= cut && bx[e] != 0u && d0 + x * 128 + lane * 4 + e < seg.doc_count) todo |= 1u << (x * 4 + e);
+        }
+        while (__any_sync(0xFFFFFFFFu, todo != 0u)) {
+          const uint32_t el = todo ? __ffs(todo) - 1 : 0u;
+          const bool had = todo != 0u;
+          todo &= todo - 1u;
+          uint32_t bits = 0u;
+#pragma unroll
+          for (int x = 0; x < 4; x++) {
+            if (el == (uint32_t)x * 4 + 0) bits = __float_as_uint(v[x].x);
+            if (el == (uint32_t)x * 4 + 1) bits = __float_as_uint(v[x].y);
+            if (el == (uint32_t)x * 4 + 2) bits = __float_as_uint(v[x].z);
+            if (el == (uint32_t)x * 4 + 3) bits = __float_as_uint(v[x].w);
+          }
+          const uint32_t doc = d0 + (el >> 2) * 128 + lane * 4 + (el & 3u);
+          cut = cut_from(wc.thr);
+          const bool pass = had && bits >= cut;
+          if (!__any_sync(0xFFFFFFFFu, pass)) continue;
+          float s = __uint_as_float(bits);
+          if (cq.nsp) {
+            uint32_t holders = 0u;
+            s = verify_doc(seg, wb, qts, nt, pass, doc, holders);  // (a sparse list the scan dropped may hold the doc)
+          }
+          wc.offer(seg, wb, cq.qi, cq.filter, pass, doc, s);
+        }
+        if (lane == 0 && wc.thr != kThrInit) atomicMax(&s_thr, wc.thr);
+      }
+    }
+    wc.merge(wb, cq.qi);  // (the query's other CTAs see the k-th key from here on)
+    if (lane == 0 && wc.thr != kThrInit) atomicMax(&s_thr, wc.thr);
+  }
+  if (sd.counters) {
+    if (lane == 0 && n_scored) atomicAdd(sd.counters + 2, (unsigned long long)n_scored);
+    if (threadIdx.x == 0 && s_open) atomicAdd(sd.counters + 1, (unsigned long long)s_open);
+  }
 }
 
 // per query slot: the scanned pairs with their bounds.  Thread per query.

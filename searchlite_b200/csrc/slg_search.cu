@@ -536,8 +536,9 @@ struct SegmentRun {
     const size_t budget = ix->smem_optin > fixed + reserve ? ix->smem_optin - fixed - reserve : 0;
     sdv.col_resident = (uint32_t)std::min<size_t>(s->n_cols, budget / (2 * kColBlock * 4));
     if (prune) {
-      // few queries keep an essential column term: one warp per (query, slice of the doc range), blocks skipped by col_tmax
-      SLG_CUDA(ix, launch_columns_pruned(pools, s->dev, wb, sdv, (int)((bt->Q * kColSlices + 7) / 8), st));
+      // few queries keep an essential column term: kColParts CTAs per query, blocks in descending order of their col_tmax bound
+      sdv.ut_max = bt->ut_max;
+      SLG_CUDA(ix, launch_columns_ordered(pools, s->dev, wb, sdv, (int)(bt->Q * kColParts), st));
     } else {
       // one CTA per SM: as many columns of a block resident in shared memory (double buffered) as fit
       const uint32_t n_cblocks = (s->doc_count + kColBlock - 1) / kColBlock;

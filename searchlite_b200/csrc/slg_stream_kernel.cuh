@@ -67,7 +67,9 @@ struct StreamDev {
   uint32_t col_resident; // columns of a block the column pass keeps in shared memory (per buffer)
   uint32_t n_smax;       // block maxima kept in shared memory (min(columns of the segment, kColMaxSlots))
   uint32_t strict;       // 1: accumulate every posting per doc (option strict_accumulate); 0: bounded accumulation, see sparse_sub_bounded
-  unsigned long long *counters;  // [4] sparse postings visited, (query, column block) pairs looked at per doc, (query, column block) pairs scored, sparse items
+  const float *ut_max;   // pruned: [U] largest unit-weight contribution of each unique term of the batch
+  unsigned long long *counters;  // [4] sparse postings visited, (query, column block) pairs looked at per doc, (query, column block) pairs scored, sparse items.
+                                 // Pruned: [1] (query, 512-doc block) pairs whose bound reached the k-th score the pass started from, [2] of those read
 };
 
 // ---- the batch's column terms: used columns -> slots, queries with a column term -> ColQ (one CTA) -------------
